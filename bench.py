@@ -10,6 +10,7 @@ whole path over the rank's shard.  Inputs are far larger than L2 (126 MB), so no
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            product arm (one process per GPU under torchrun)
   python bench.py --impl reference ...                           the reference's own CPU path (oracle/_ref) on the host cores
+  python bench.py ... --dump-outputs DIR                         also write what the last timed step computed (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -99,6 +100,26 @@ class ClockSampler:
 def make_segment(period):
     from sdvpcmdecoder_b200 import synth
     return synth.make_stc007(period, seed=1234, periodic=True)
+
+
+DUMP_BYTES = 60_000_000      # all files of one --dump-outputs run together (headers aside), under 64 MB
+
+
+def dump_outputs(out_dir, samples, flags, first_block, rank, world):
+    """Write what a caller of the decode path receives -- the samples [nb, 6] (int16) and the sample flags [nb, 6] -- as float32
+    .npy files, with the global index of every block as float64.  A tape too large for DUMP_BYTES is represented by a fixed
+    sample of its blocks (seeded, so two runs with the same arguments write the same blocks).  Under torchrun every rank writes
+    its own shard's files, named *.rank<r>.npy."""
+    import torch
+    nb = samples.shape[0]
+    k = min(nb, DUMP_BYTES // world // (6 * 4 * 2 + 8))
+    rows = np.arange(nb) if k == nb else np.sort(np.random.default_rng(1234 + rank).choice(nb, k, replace=False))
+    idx = torch.from_numpy(rows).to(samples.device)
+    suffix = "" if world == 1 else f".rank{rank}"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"samples{suffix}.npy"), samples[idx].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, f"flags{suffix}.npy"), flags[idx].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, f"block_index{suffix}.npy"), (rows + first_block).astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ reference arm / CPU baseline
@@ -344,6 +365,7 @@ def main():
     ap.add_argument("--fuse", action="store_true", help="finish the in-frame data blocks inside the bulk pass (sdv_stc007_fuse_next_decode; slower, see DESIGN 3.3)")
     ap.add_argument("--no-lazy", action="store_true", help="wait for the bulk pass inside every decode call (no lazy verification)")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the process to the GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the samples and flags of the last one to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)
@@ -460,6 +482,8 @@ def main():
     launches_timed = int(tm["kernel_launches"])
     stats = v2d.stats()
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, samples, flags, sharding.first_block(F, rank, world, LPF), rank, world)
 
     # ---- the same K steps without the warm start (a one-shot decode of a tape is a cold call on every GPU)
     v2d.warm_start = False

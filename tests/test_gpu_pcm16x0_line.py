@@ -1,16 +1,15 @@
-"""PCM-16x0 line decode on the GPU (through the C ABI) against the compiled reference (oracle/_ref) and the golden fixture."""
+"""PCM-16x0 line decode on the GPU (through the C ABI) against the reference's sub-line records and sample streams (stored in
+tests/golden/reference_streams.json) and the golden fixture."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle import refbind as R
 from sdvpcmdecoder_b200 import synth, capi
 from sdvpcmdecoder_b200.capi import LINE_REC, LINE_AUX
 from tests import util
 
 pytestmark = pytest.mark.gpu
-have_ref = pytest.mark.skipif(not R.available(), reason="oracle/_ref not built")
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
@@ -34,56 +33,91 @@ def _decode(ctx, luma, mode=2, dup=True):
 
 
 def _check(ctx, luma, mode=2, dup=True):
-    ref = R.v2d_run(R.TYPE_PCM16X0, mode, luma, line_dup=dup)
-    ref = ref[ref["service_type"] == 0][:luma.shape[0] * luma.shape[1] * 3]
+    """The product's three sub-line records of every line equal the reference's (VideoToDigital, the part of the line
+    included); -> (records, stats)."""
     rec, aux, st = _decode(ctx, luma, mode, dup)
-    bad = util.compare_line_records(util.x0_ref_to_product(ref), rec, aux, oracle_only_flags=0)
-    if not np.array_equal(ref["line_part"], rec["reserved"]):
-        bad.append("line_part")
+    bad = util.lines_mismatch("pcm16x0_lines", luma, (mode, dup), rec, aux, with_part=True)
     assert not bad, bad
-    return ref, st
+    return rec, st
 
 
-@have_ref
+# the tapes of the line tests: (luma, mode, dup) lists, shared with tests/golden/make_golden.py
+def clean_tape():
+    return synth.make_pcm16x0(10)["luma"]
+
+
+def drift_tape():
+    a = synth.make_pcm16x0(3, seed=1)["luma"]
+    b = synth.make_pcm16x0(3, seed=2, x0=9, x1=713)["luma"]
+    return np.concatenate([a, b, a[:2]])
+
+
+def damaged_runs(mode):
+    base = synth.make_pcm16x0(2)["luma"]
+    return [(t, mode, True) for t in (
+        base,
+        synth.damage_stc007(base, seed=100 + mode),
+        synth.damage_stc007(base, seed=200 + mode, jitter=False, blur=False, sigma=25., dropout_frac=0.05),
+        synth.make_pcm16x0(2, seed=11, x0=-5, x1=710)["luma"],
+        synth.make_pcm16x0(2, seed=12, x0=6, x1=723)["luma"],
+        synth.damage_stc007(synth.make_pcm16x0(2, seed=13, x0=-7, x1=725)["luma"], seed=5, jitter=False, blur=False, sigma=6., dropout_frac=0.02),
+        synth.make_pcm16x0(1, seed=15, width=1440)["luma"])]
+
+
+def sparse_tape():
+    luma = synth.make_pcm16x0(8, seed=5)["luma"].copy()
+    luma[3, 100:104, 200:500] = 255
+    luma[6, 0, :] = 16
+    return luma
+
+
+def insane_runs():
+    base = synth.make_pcm16x0(1)["luma"]
+    return [(base[:, :64], 3, True), (synth.damage_stc007(base, seed=102)[:, :64], 3, True)]
+
+
+WIDTHS = [640, 1024, 1920]
+
+
+def width_runs(width):
+    luma = synth.make_pcm16x0(3, seed=width, width=width)["luma"]
+    return [(luma, 2, True), (synth.damage_stc007(luma[:2], seed=width + 1, sigma=6.0, dropout_frac=0.03, jitter=False, blur=False), 2, True)]
+
+
+def line_runs():
+    runs = [(clean_tape(), 2, dup) for dup in (True, False)] + [(drift_tape(), 2, dup) for dup in (True, False)]
+    runs += [(sparse_tape(), 2, True)] + insane_runs()
+    for mode in (0, 1, 2):
+        runs += damaged_runs(mode)
+    for w in WIDTHS:
+        runs += width_runs(w)
+    return runs
+
+
 def test_clean_tape_all_fields_and_bulk_path(ctx):
-    luma = synth.make_pcm16x0(10)["luma"]
+    luma = clean_tape()
     for dup in (True, False):
         ref, st = _check(ctx, luma, dup=dup)
         assert st["frames_skipped"] == 10 and st["lines_chain"] == 0, (dup, st)
     assert (ref["flags"] & 1).mean() > 0.99
 
 
-@have_ref
 def test_coordinates_drift_between_frames(ctx):
     """Frames whose prescan coordinates differ: with the duplicate-line check on the reference keeps decoding with the
     history median, without it every frame follows its own prescan."""
-    a = synth.make_pcm16x0(3, seed=1)["luma"]
-    b = synth.make_pcm16x0(3, seed=2, x0=9, x1=713)["luma"]
-    luma = np.concatenate([a, b, a[:2]])
+    luma = drift_tape()
     for dup in (True, False):
         _check(ctx, luma, dup=dup)
 
 
-@have_ref
 @pytest.mark.parametrize("mode", [0, 1, 2])
 def test_damaged_and_cut_tapes(ctx, mode):
-    base = synth.make_pcm16x0(2)["luma"]
-    _check(ctx, base, mode)
-    _check(ctx, synth.damage_stc007(base, seed=100 + mode), mode)
-    _check(ctx, synth.damage_stc007(base, seed=200 + mode, jitter=False, blur=False, sigma=25., dropout_frac=0.05), mode)
-    _check(ctx, synth.make_pcm16x0(2, seed=11, x0=-5, x1=710)["luma"], mode)
-    _check(ctx, synth.make_pcm16x0(2, seed=12, x0=6, x1=723)["luma"], mode)
-    _check(ctx, synth.damage_stc007(synth.make_pcm16x0(2, seed=13, x0=-7, x1=725)["luma"], seed=5, jitter=False, blur=False,
-                                    sigma=6., dropout_frac=0.02), mode)
-    _check(ctx, synth.make_pcm16x0(1, seed=15, width=1440)["luma"], mode)
+    for luma, m, dup in damaged_runs(mode):
+        _check(ctx, luma, m, dup)
 
 
-@have_ref
 def test_sparse_damage_mixes_bulk_and_chain(ctx):
-    luma = synth.make_pcm16x0(8, seed=5)["luma"].copy()
-    luma[3, 100:104, 200:500] = 255
-    luma[6, 0, :] = 16
-    ref, st = _check(ctx, luma)
+    ref, st = _check(ctx, sparse_tape())
     assert 0 < st["frames_skipped"] < 8 and st["lines_chain"] > 0
 
 
@@ -96,7 +130,6 @@ def test_golden_sublines(ctx):
         assert np.array_equal(g[name + "_recs"].view(LINE_REC).reshape(-1), rec), name
 
 
-@have_ref
 def test_pipeline_samples_against_reference(ctx):
     from tests.test_pcm16x0_stitch import stitch_cases, ref_pairs, frames_match
     h, ops, torch = ctx
@@ -135,11 +168,10 @@ def test_config3_round_trip(ctx):
     assert st["frames_skipped"] == 1000 and st["lines_chain"] == 0
 
 
-@have_ref
 def test_mode_insane_reference_level_sweep(ctx):
-    base = synth.make_pcm16x0(1)["luma"]
-    _check(ctx, base[:, :64], mode=3)
-    ref, st = _check(ctx, synth.damage_stc007(base, seed=102)[:, :64], mode=3)
+    (a, ma, da), (b, mb, db) = insane_runs()
+    _check(ctx, a, ma, da)
+    ref, st = _check(ctx, b, mb, db)
     assert ((ref["flags"] >> 5) & 1).sum() > 0
 
 
@@ -157,12 +189,10 @@ def test_host_buffer_entry_points(ctx):
     assert valid.mean() > 0.97 and np.array_equal(smp[valid], src[valid])
 
 
-@have_ref
-@pytest.mark.parametrize("width", [640, 1024, 1920])
+@pytest.mark.parametrize("width", WIDTHS)
 def test_frame_widths(ctx, width):
-    luma = synth.make_pcm16x0(3, seed=width, width=width)["luma"]
-    _check(ctx, luma)
-    _check(ctx, synth.damage_stc007(luma[:2], seed=width + 1, sigma=6.0, dropout_frac=0.03, jitter=False, blur=False))
+    for luma, m, dup in width_runs(width):
+        _check(ctx, luma, m, dup)
 
 
 def test_frame_info_control_bits(ctx):
@@ -188,7 +218,7 @@ def test_own_alignment_equals_reference_pipeline(ctx):
     (padding sweep on the device, findSIPadding's decisions on the host) -- the reference's PCMSamplePair stream frame by frame,
     on configs 3 / 3B, damaged tapes and vertically shifted captures; and the host build of the same code gives the same
     alignment records."""
-    from tests.test_pcm16x0_stitch import alignment_cases, ref_pairs
+    from tests.test_pcm16x0_stitch import alignment_cases, ref_pairs, pairs_mismatch
     h, ops, torch = ctx
     for name, luma in alignment_cases().items():
         v2d = ops.VideoToDigital(h)
@@ -201,7 +231,7 @@ def test_own_alignment_equals_reference_pipeline(ctx):
             smp, fl, al = st.doFrameReassembleAuto(recs, n, luma.shape[1])
             torch.cuda.synchronize()
             ref = ref_pairs(luma, bff, p_corr)
-            assert np.array_equal(ref[0], smp.cpu().numpy()) and np.array_equal(ref[1], fl.cpu().numpy()), (name, bff, p_corr, al)
+            assert not pairs_mismatch(ref, smp.cpu().numpy(), fl.cpu().numpy()), (name, bff, p_corr, pairs_mismatch(ref, smp.cpu().numpy(), fl.cpu().numpy()), al)
             es, ef, eal = util.emu_x0_stitch_auto(ops.records_to_numpy(recs, LINE_REC), n, luma.shape[1], bff, p_corr=p_corr)
             assert np.array_equal(al, eal), (name, bff, p_corr)
 
@@ -211,7 +241,7 @@ def test_ei_stitching_equals_reference_pipeline(ctx):
     frame on the device, findEIFrameStitching's decisions in the library -- the reference's PCMSamplePair stream with
     setFormat(FORMAT_EI) frame by frame, on every tape of ei_cases(); the host build gives the same alignment records; the
     padding history carries over calls (file_start = 0) and is dropped by a change of format."""
-    from tests.test_pcm16x0_stitch import ei_cases, ref_pairs
+    from tests.test_pcm16x0_stitch import ei_cases, ref_pairs, pairs_mismatch
     h, ops, torch = ctx
     for name, luma in ei_cases().items():
         v2d = ops.VideoToDigital(h)
@@ -224,7 +254,7 @@ def test_ei_stitching_equals_reference_pipeline(ctx):
             smp, fl, al = st.doFrameReassembleAuto(recs, n, luma.shape[1])
             torch.cuda.synchronize()
             ref = ref_pairs(luma, bff, p_corr, ei=True)
-            assert np.array_equal(ref[0], smp.cpu().numpy()) and np.array_equal(ref[1], fl.cpu().numpy()), (name, bff, p_corr, al)
+            assert not pairs_mismatch(ref, smp.cpu().numpy(), fl.cpu().numpy()), (name, bff, p_corr, pairs_mismatch(ref, smp.cpu().numpy(), fl.cpu().numpy()), al)
             es, ef, eal = util.emu_x0_stitch_auto(ops.records_to_numpy(recs, LINE_REC), n, luma.shape[1], bff, p_corr=p_corr, ei=True)
             assert np.array_equal(al, eal), (name, bff, p_corr)
             if name in ("clean", "shift3") and p_corr:
@@ -232,7 +262,7 @@ def test_ei_stitching_equals_reference_pipeline(ctx):
                 assert (al["cut_lines"] == 0).all() and (al["mask_seams"] == 0).all()
                 st.setTopPadding(int(al["top_padding"][0][0]), int(al["top_padding"][0][1]))
                 ps, pf = st.doFrameReassemble(recs, n, luma.shape[1])
-                assert np.array_equal(ref[0], ps.cpu().numpy()) and np.array_equal(ref[1], pf.cpu().numpy()), (name, bff, "preset EI")
+                assert not pairs_mismatch(ref, ps.cpu().numpy(), pf.cpu().numpy()), (name, bff, "preset EI")
             if name in ("shift50", "blanked_shift-20") and not bff and p_corr:
                 # two calls of two frames = one call of four (the history of accepted paddings stays on the handle) ...
                 rl = ops.records_to_numpy(recs, LINE_REC).reshape(n, -1)
@@ -240,7 +270,7 @@ def test_ei_stitching_equals_reference_pipeline(ctx):
                 for k, fs in ((0, True), (2, False)):
                     part = torch.from_numpy(np.ascontiguousarray(rl[k:k + 2]).view(np.uint8)).cuda()
                     halves.append(st.doFrameReassembleAuto(part, 2, luma.shape[1], file_start=fs))
-                assert np.array_equal(np.concatenate([x[0].cpu().numpy() for x in halves]), ref[0]), name
+                assert np.array_equal(np.concatenate([x[0].cpu().numpy() for x in halves]), smp.cpu().numpy()), name      # = the reference's
                 assert np.array_equal(np.concatenate([x[2] for x in halves]), al), name
                 # ... and an SI call in between drops it
                 st.setFormat(st.FORMAT_SI)

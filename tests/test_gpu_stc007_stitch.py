@@ -1,12 +1,11 @@
 """GPU parity of sdv_stc007_stitch_frames (through the C ABI) with the UNMODIFIED reference pipeline: the product's
-PCMSamplePair stream (l, r, three flags per sample) and its data blocks against VideoToDigital + STC007DataStitcher of
-oracle/_ref on the same tapes.  Run on the B200 box."""
+PCMSamplePair stream (l, r, three flags per sample) and its data blocks against those stored for VideoToDigital +
+STC007DataStitcher on the same tapes (tests/golden/reference_streams.json; provenance in make_golden.streams_golden).  Needs a GPU."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle import refbind as R
 from sdvpcmdecoder_b200 import synth, capi
 from sdvpcmdecoder_b200.capi import LINE_REC, BLOCK_REC
 from tests import util
@@ -47,10 +46,33 @@ def test_sample_stream_equals_reference_pipeline(ctx, name):
         assert (blocks["flags"] & capi.BF_UNSAFE).any() and (blocks["flags"] & 2).any() and not (info["flags"] & (capi.FA_MASK_INNER | capi.FA_MASK_PREV_OUTER)).any()
 
 
-@pytest.mark.parametrize("seed", [4567, 4568, 4569, 4570, 4571])
+CONFIG4_SEEDS = [4567, 4568, 4569, 4570, 4571]
+
+
+def config4_tape(seed):
+    return synth.damage_stc007(synth.make_stc007(24, seed=seed - 4000)["luma"], seed=seed)
+
+
+def two_shard_tape():
+    luma = synth.damage_stc007(synth.make_stc007(12, seed=441)["luma"], seed=442)        # BASELINE config 4 damage
+    # BROKEN blocks just ahead of the boundary: lines with a valid CRC and foreign words (a splice) at the end of frame 5,
+    # shard 0's last; the 128-block window they open reaches two blocks into shard 1
+    luma[5, 561:576:2] = luma[4, 101:116:2]
+    return luma
+
+
+def ntsc16_tape():
+    return synth.damage_stc007(synth.make_stc007(6, seed=441, pal=False, f1_16bit=True)["luma"], seed=442, **HEAVY)
+
+
+def cwd_config4_tape():
+    return synth.damage_stc007(synth.make_stc007(24, seed=567)["luma"], seed=4567)
+
+
+@pytest.mark.parametrize("seed", CONFIG4_SEEDS)
 def test_config4_sample_stream(ctx, seed):
     """BASELINE config 4 (damage_stc007 with its default mix) on 24 PAL frames, plain STC-007, PAL / TFF / 14-bit preset."""
-    luma = synth.damage_stc007(synth.make_stc007(24, seed=seed - 4000)["luma"], seed=seed)
+    luma = config4_tape(seed)
     pairs, ref_blocks = reference_stream(luma, 1, 1, 1, 1, 1)
     blocks, samples, flags, info, _, _ = _product(ctx, luma, 1, 1)
     assert not stream_mismatch(pairs, samples, flags)
@@ -154,10 +176,7 @@ def test_two_shards_on_a_damaged_tape_equal_the_reference(ctx):
     group) -- against the reference pipeline's PCMSamplePair stream of the UNSHARDED damaged tape."""
     import torch
     from sdvpcmdecoder_b200 import operators as ops, sharding
-    luma = synth.damage_stc007(synth.make_stc007(12, seed=441)["luma"], seed=442)        # BASELINE config 4 damage
-    # BROKEN blocks just ahead of the boundary: lines with a valid CRC and foreign words (a splice) at the end of frame 5,
-    # shard 0's last; the 128-block window they open reaches two blocks into shard 1
-    luma[5, 561:576:2] = luma[4, 101:116:2]
+    luma = two_shard_tape()
     pairs, ref_blocks = reference_stream(luma, 1, 1, 1, 1, 1)
     H, world = luma.shape[1], 2
     out_s, out_f, states, handles, stitchers, recs_all, halos = [], [], [], [], [], [], []
@@ -212,7 +231,7 @@ def test_detected_audio_resolution(ctx):
         assert not stream_mismatch(pairs, samples, flags), name
         assert not block_mismatch(ref_blocks, blocks), name
     # everything detected at once (video standard, field order, resolution) on an NTSC 16-bit tape
-    n16 = synth.damage_stc007(synth.make_stc007(6, seed=441, pal=False, f1_16bit=True)["luma"], seed=442, **HEAVY)
+    n16 = ntsc16_tape()
     pairs, ref_blocks = reference_stream(n16, 0, 0, 0, 1, 1)
     blocks, samples, flags, info, _, _ = _product_auto_res(ctx, n16, std=0, order=0)
     assert not stream_mismatch(pairs, samples, flags) and not block_mismatch(ref_blocks, blocks)
@@ -263,7 +282,7 @@ def test_cwd_sample_stream_equals_reference_pipeline(ctx):
 
 
 def test_cwd_config4_24_frames(ctx):
-    luma = synth.damage_stc007(synth.make_stc007(24, seed=567)["luma"], seed=4567)
+    luma = cwd_config4_tape()
     pairs, ref_blocks = reference_stream(luma, 1, 1, 1, 1, 1, cwd=1)
     blocks, samples, flags, info, _, _ = _product_cwd(ctx, luma, 1, 1, 1, 1, 1)
     assert not stream_mismatch(pairs, samples, flags)

@@ -56,8 +56,8 @@ def test_m2_on_host_against_reference_live():
 
 
 @pytest.mark.gpu
-@have_ref
 def test_m2_gpu_against_reference():
+    """The GPU path against the reference's line records and PCMSamplePair stream (tests/golden/reference_streams.json)."""
     import torch
     from sdvpcmdecoder_b200 import operators as ops
     h = capi.Handle(0)
@@ -69,10 +69,7 @@ def test_m2_gpu_against_reference():
         st.setM2SampleFormat(True)
         _, samples, flags = st.doFrameReassemble(recs, luma.shape[0], luma.shape[1])
         torch.cuda.synchronize()
-        bad = util.compare_line_records(ref_lines(luma, R.TYPE_M2), ops.records_to_numpy(recs, LINE_REC), ops.records_to_numpy(aux, LINE_AUX))
+        bad = util.lines_mismatch("m2_lines", luma, (), ops.records_to_numpy(recs, LINE_REC), ops.records_to_numpy(aux, LINE_AUX))
         assert not bad, (name, bad)
-        p = ref_pairs(luma)
-        s, f = samples.cpu().numpy().reshape(-1, 2), flags.cpu().numpy().reshape(-1, 2)
-        assert len(p) == len(s)
-        assert np.array_equal(p["l"], s[:, 0]) and np.array_equal(p["r"], s[:, 1]), name
-        assert np.array_equal(p["flags_l"] & 7, f[:, 0]) and np.array_equal(p["flags_r"] & 7, f[:, 1]), name
+        bad = util.stream_mismatch_digests(util.golden_stream("m2", luma, ()), [samples.cpu().numpy().reshape(-1, 2), flags.cpu().numpy().reshape(-1, 2)])
+        assert not bad, (name, bad)

@@ -2,21 +2,21 @@
 chain, frame assembly, seam masking and the broken-block countdown.
 
 CPU part: the library's host decision chain (csrc/stc007_stitch_host.h) and the SDV_HD device code (csrc/stc007_stitch.cuh),
-built as host code by tests/hostemu, against the PCMSamplePair stream and the data blocks of the UNMODIFIED reference
-pipeline (oracle/_ref, VideoToDigital + STC007DataStitcher) on the same tapes -- damaged far beyond BASELINE config 4, shifted
-vertically, with blank and partial frames, with field order / video standard preset or detected.  GPU part
-(tests/test_gpu_stc007_stitch.py): the CUDA path through the C ABI against the same reference streams.
+built as host code by tests/hostemu and fed with the oracle's line records, against the PCMSamplePair streams and data blocks
+stored for these tapes in tests/golden/reference_streams.json -- damaged far beyond BASELINE config 4, shifted vertically, with
+blank and partial frames, with field order / video standard preset or detected.  The stored streams stand for the reference
+pipeline's (VideoToDigital + STC007DataStitcher) output; tests/golden/make_golden.py streams_golden() says where they come from
+and what ties them to the reference.  GPU part (tests/test_gpu_stc007_stitch.py): the CUDA path through the C ABI against the
+same streams.
 """
 import os
 
 import numpy as np
 import pytest
 
-from oracle import refbind as R
 from sdvpcmdecoder_b200 import synth, capi
 from tests import util
 
-needs_ref = pytest.mark.skipif(not R.available(), reason="oracle/_ref not built")
 HEAVY = dict(sigma=20.0, dropout_frac=0.1, marker_kill_frac=0.05)
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "stc007_stitch.npz")
 
@@ -63,36 +63,43 @@ def stitch_cases():
     return c
 
 
+BLOCKS_PER_FRAME = 588          # 2 x 294 assembled lines (PAL), one data block each: the unit of the stored digests
+
+
 def reference_stream(luma, std, order, res, p, q, cwd=0):
-    cfg = R.StitchCfg()
-    cfg.video_std, cfg.field_order, cfg.resolution, cfg.p_corr, cfg.q_corr, cfg.cwd = std, order, res, p, q, cwd
-    pairs, _, blocks = R.pipeline_run(R.TYPE_STC007, R.MODE_NORMAL, luma, cfg)
-    return pairs[pairs["service_type"] == 0], blocks
+    """The stored PCMSamplePair stream (l, r, flags & 7) and data blocks of VideoToDigital + STC007DataStitcher on this tape with
+    these settings (tests/golden/reference_streams.json; provenance in make_golden.streams_golden)."""
+    g = util.golden_stream("stc007", luma, (std, order, res, p, q, cwd))
+    return g["pairs"], g["blocks"]
+
+
+def pair_arrays(samples, flags):
+    return samples.reshape(-1, 2), flags.reshape(-1, 2)
+
+
+def block_arrays(blocks):
+    return [blocks[n] for n in ("words", "line_crc", "word_valid", "audio_state", "resolution")] + [blocks["flags"] & 0x1F]
 
 
 def stream_mismatch(pairs, samples, flags):
-    got, gf = samples.reshape(-1, 2), flags.reshape(-1, 2)
-    if len(got) != len(pairs):
-        return f"{len(got)} pairs, reference {len(pairs)}"
-    d = (pairs["l"] != got[:, 0]) | (pairs["r"] != got[:, 1]) | ((pairs["flags_l"] & 7) != gf[:, 0]) | ((pairs["flags_r"] & 7) != gf[:, 1])
-    return f"{int(d.sum())} pairs differ, first blocks {np.unique(np.nonzero(d)[0] // 3)[:6]}" if d.any() else ""
+    return util.stream_mismatch_digests(pairs, pair_arrays(samples, flags))
 
 
 def block_mismatch(ref_blocks, blocks):
-    if len(ref_blocks) != len(blocks):
-        return f"{len(blocks)} blocks, reference {len(ref_blocks)}"
-    bad = [n for n in ("words", "line_crc", "word_valid", "audio_state", "resolution") if not np.array_equal(ref_blocks[n], blocks[n])]
-    if not np.array_equal(ref_blocks["flags"] & 0x1F, blocks["flags"] & 0x1F):
-        bad.append("flags")
-    return ", ".join(bad)
+    return util.stream_mismatch_digests(ref_blocks, block_arrays(blocks))
 
 
-@needs_ref
+def oracle_lines(luma):
+    """Line records of the oracle's VideoToDigital (equal to the reference's: tests/test_oracle.py) for the host-built stitcher."""
+    from oracle import oraclebind as O
+    return util.lines_from_oracle(O.v2d_stc007(capi.MODE_NORMAL, luma, True))
+
+
 @pytest.mark.parametrize("name", sorted(stitch_cases()))
 def test_host_chain_and_device_logic_against_reference_pipeline(name):
     luma, std, order, res, p, q = stitch_cases()[name]
     pairs, ref_blocks = reference_stream(luma, std, order, res, p, q)
-    recs = util.lines_from_oracle(util.ref_lines_in_frame_order(R.v2d_run(R.TYPE_STC007, R.MODE_NORMAL, luma), keep=(0, 7)))
+    recs = oracle_lines(luma)
     blocks, samples, flags, info = util.emu_stc007_stitch(recs, luma.shape[0], luma.shape[1], video_std=std, field_order=order, res16=(res == 2),
                                                           p_corr=bool(p), q_corr=bool(q))
     assert not stream_mismatch(pairs, samples, flags)
@@ -153,14 +160,13 @@ CPU_RESOLUTION_CASES = ["clean16", "heavy16", "switch_14_to_16", "blank_frames_1
 CPU_CWD_CASES = ["config4", "heavy", "dropouts16", "heavy16_auto_res", "p_only", "sparse"]
 
 
-@needs_ref
 @pytest.mark.parametrize("name", CPU_RESOLUTION_CASES)
 def test_detected_audio_resolution_against_reference_pipeline(name):
     """getFieldResolution + detectAudioResolution + getDataBlockResolution: the resolution is not preset, every block and every
     seam takes the mode of the fields it touches."""
     luma = resolution_cases()[name]
     pairs, ref_blocks = reference_stream(luma, 1, 1, 0, 1, 1)
-    recs = util.lines_from_oracle(util.ref_lines_in_frame_order(R.v2d_run(R.TYPE_STC007, R.MODE_NORMAL, luma), keep=(0, 7)))
+    recs = oracle_lines(luma)
     blocks, samples, flags, info = util.emu_stc007_stitch(recs, luma.shape[0], luma.shape[1], video_std=1, field_order=1, res16=None)
     assert not stream_mismatch(pairs, samples, flags)
     assert not block_mismatch(ref_blocks, blocks)
@@ -190,14 +196,13 @@ def cwd_cases():
     return c
 
 
-@needs_ref
 @pytest.mark.parametrize("name", CPU_CWD_CASES)
 def test_cwd_against_reference_pipeline(name):
     """performCWD + the deinterleaver's CWD stage: the PCMSamplePair stream and the data blocks of the reference pipeline with
     setCWDCorrection(true)."""
     luma, std, order, res, p, q = cwd_cases()[name]
     pairs, ref_blocks = reference_stream(luma, std, order, res, p, q, cwd=1)
-    recs = util.lines_from_oracle(util.ref_lines_in_frame_order(R.v2d_run(R.TYPE_STC007, R.MODE_NORMAL, luma), keep=(0, 7)))
+    recs = oracle_lines(luma)
     blocks, samples, flags, info = util.emu_stc007_stitch(recs, luma.shape[0], luma.shape[1], video_std=std, field_order=order,
                                                           res16={0: None, 1: False, 2: True}[res], p_corr=bool(p), q_corr=bool(q), cwd=True)
     assert not stream_mismatch(pairs, samples, flags)

@@ -2,6 +2,8 @@
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -13,7 +15,57 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 EMU_SRC = os.path.join(HERE, "hostemu", "hostemu.cpp")
 EMU_LIB = os.path.join(HERE, "hostemu", "_build", "libhostemu.so")
+REF_STREAMS = os.path.join(HERE, "golden", "reference_streams.json")
 _emu = None
+_ref_streams = None
+
+
+# ---- the reference pipeline's output streams, stored as digests (tests/golden/reference_streams.json, make_golden.py streams)
+def tape_key(kind, luma, params):
+    """Key of one reference run: the tape's bytes, its shape and the pipeline settings."""
+    h = hashlib.blake2b(np.ascontiguousarray(luma).tobytes(), digest_size=16)
+    h.update(repr((kind, tuple(luma.shape), tuple(int(p) for p in params))).encode())
+    return h.hexdigest()
+
+
+def chunk_digests(arrays, rows):
+    """blake2b digest of every [rows] rows of the arrays (all of one length), in order: one digest per frame."""
+    n = len(arrays[0])
+    assert all(len(a) == n for a in arrays)
+    out = []
+    for a in range(0, n, rows):
+        h = hashlib.blake2b(digest_size=16)
+        for x in arrays:
+            h.update(np.ascontiguousarray(x[a:a + rows]).tobytes())
+        out.append(h.hexdigest())
+    return out
+
+
+def stream_entry(arrays, rows):
+    """Stored form of a stream: a digest per frame (chunk of rows) over all arrays, and a digest per array over all frames."""
+    return {"rows": int(len(arrays[0])), "chunk": rows, "digests": chunk_digests(arrays, rows),
+            "fields": [chunk_digests([a], len(a))[0] for a in arrays]}
+
+
+def stream_mismatch_digests(ref, arrays):
+    """'' when the arrays equal the stored stream; else which frames (chunks) and which arrays (by position) differ."""
+    if len(arrays[0]) != ref["rows"]:
+        return f"{len(arrays[0])} rows, reference {ref['rows']}"
+    got = chunk_digests(arrays, ref["chunk"])
+    bad = [i for i, (a, b) in enumerate(zip(got, ref["digests"])) if a != b]
+    fields = [i for i, (a, d) in enumerate(zip(arrays, ref["fields"])) if chunk_digests([a], len(a))[0] != d]
+    return f"{len(bad)} of {len(got)} frames differ, first {bad[:6]}; arrays {fields} differ" if bad else ""
+
+
+def golden_stream(kind, luma, params):
+    """The stored reference stream(s) of this tape and these settings; a tape without one is an error, not a skip."""
+    global _ref_streams
+    if _ref_streams is None:
+        with open(REF_STREAMS) as f:
+            _ref_streams = json.load(f)
+    key = tape_key(kind, luma, params)
+    assert key in _ref_streams, f"no reference stream stored for this {kind} tape {tuple(luma.shape)} / {params} (make_golden.py streams)"
+    return _ref_streams[key]
 
 
 def build_hostemu():
@@ -111,6 +163,19 @@ def compare_line_records(oracle_recs, rec, aux=None, tier_a_only=False, oracle_o
                 d = o[n] != aux[n]
                 bad.append(f"aux.{n}: {int(d.sum())} lines, first {np.nonzero(d)[0][:5]}")
     return bad
+
+
+def line_arrays(rec, aux, with_part=False):
+    """The fields compare_line_records looks at, of product records + aux (with_part: the PCM-16x0 sub-line part in reserved),
+    in the order the stored digests of reference line records use (tests/golden/reference_streams.json): words, flags,
+    REC_FIELDS[1:], mark_stages, AUX_FIELDS[, reserved]."""
+    a = [rec["words"], rec["flags"]] + [rec[n] for n in REC_FIELDS[1:]] + [rec["mark_stages"]] + [aux[n] for n in AUX_FIELDS]
+    return a + [rec["reserved"]] if with_part else a
+
+
+def lines_mismatch(kind, luma, params, rec, aux, with_part=False):
+    """'' when the product's line records equal the reference's stored for this tape (one digest per frame)."""
+    return stream_mismatch_digests(golden_stream(kind, luma, params), line_arrays(rec, aux, with_part))
 
 
 def lines_from_oracle(o):
