@@ -47,18 +47,6 @@ __global__ void __launch_bounds__(P1S_THREADS, 5) pcm16x0_prescan_kernel(const u
     }
 }
 
-struct X0BulkParams
-{
-    const u8 *luma; int H, W; size_t stride;
-    int n_frames;
-    const P1Preset *presets;
-    int line_dup, mode;
-    sdv_line_rec *recs; sdv_line_aux *aux;     // [n_frames*H*3]
-    u8 *clean;
-    u32 *frame_bw;                  // black | white<<8 the last lines of the frame were given
-    int use_tma, warps; u32 slot_bytes;
-};
-
 // Black/white levels of one staged row (findPCM16X0BW + findBlackWhite tail), by one warp.
 __device__ __forceinline__ u32 x0_warp_black_white(const u8 *row, int W, u32 *hist, int lane)
 {
@@ -105,48 +93,20 @@ __device__ __forceinline__ u32 x0_picked_counts(Ppb pp, int mode, int W)
     return l|((u32)t.picked_right<<4);
 }
 
-__global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(const __grid_constant__ X0BulkParams p)
+__global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(const __grid_constant__ P1BulkParams p)
 {
     extern __shared__ __align__(128) u8 dsm[];
-    u64 *bars = (u64 *)dsm;
-    u16 *crc_tab = (u16 *)(dsm+128);
+    u16 *crc_tab = (u16 *)(dsm+BULK_BAR_BYTES);
     const int warp = threadIdx.x>>5, lane = threadIdx.x&31;
-    u32 *hist = (u32 *)(dsm+128+512)+warp*256;
-    const u32 stage_bytes = BULK_ROWS*p.slot_bytes;
-    u8 *ring = dsm+P1_BULK_HEADER+(size_t)warp*BULK_STAGES*stage_bytes;
-    u64 *bar = bars+warp*BULK_STAGES;
+    u32 *hist = (u32 *)(dsm+BULK_BAR_BYTES+512)+warp*256;
     for(int i=threadIdx.x;i<256;i+=blockDim.x) crc_tab[i] = c_crc8[i];
-    if(p.use_tma&&(lane==0))
-    {
-        for(int s=0;s<BULK_STAGES;s++) mbar_init(&bar[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    BulkRing rb(dsm, P1_BULK_HEADER, p.luma, p.H, p.W, p.stride, 0, p.n_frames, p.use_tma, p.warps, p.slot_bytes);
     __syncthreads();
+    rb.prime();
 
     const int hf = p.H/2;
-    const int nbatch = (p.H+BULK_ROWS-1)/BULK_ROWS;
-    const long long n_units = p.n_frames;
-    const long long gw = (long long)blockIdx.x*p.warps+warp, gstride = (long long)gridDim.x*p.warps;
-    const long long my_units = (gw<n_units) ? ((n_units-gw+gstride-1)/gstride) : 0;
-    const long long n_items = my_units*nbatch;
     const int fld = lane&1;
     const int pixel_stop = p.W-1;
-
-    auto issue = [&](long long it)
-    {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int r0 = (int)(it%nbatch)*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int s = (int)(it&1);
-        if(lane==0)
-        {
-            const u32 bytes = (u32)rows*(u32)p.stride;
-            mbar_expect_tx(&bar[s], bytes);
-            bulk_g2s(smem_u32(ring)+(u32)s*stage_bytes, p.luma+((size_t)u*p.H+(size_t)r0)*p.stride, bytes, &bar[s]);
-        }
-        __syncwarp();
-    };
-    if(p.use_tma) { if(n_items>0) issue(0); if(n_items>1) issue(1); }
 
     // the running coordinates of the tape (duplicate-line check on): those of the first frame
     const P1Preset ps0 = p.presets[0];
@@ -162,18 +122,13 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(cons
     Ppb fpp = gpp; Coord fc = gc; u32 f_picked = g_picked;      // coordinates of the frame's first line / of the whole frame (no dup check)
     u32 bw0 = 0, bwb = 0, bwc = 0;
 
-    for(long long it=0;it<n_items;it++)
+    for(long long it=0;it<rb.n_items;it++)
     {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int b = (int)(it%nbatch), r0 = b*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int f = (int)u;
-        const int s = (int)(it&1);
+        const BulkItem t = rb.item(it);
+        const int f = t.f, b = t.b, r0 = t.r0, rows = t.rows;
         const int k = (r0>>1)+(lane>>1);
         const int frow = r0+lane;
         const bool active = lane<rows;
-        const u8 *stage = ring+(size_t)s*stage_bytes;
-        const u8 *row = stage+(size_t)lane*p.slot_bytes;
         if(b==0)
         {
             const P1Preset ps = p.presets[f];
@@ -186,18 +141,8 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(cons
             f_picked = x0_picked_counts(fpp, p.mode, p.W);
             for(int q=0;q<3;q++) cw[q][0] = cw[q][1] = 0;
         }
-        if(p.use_tma) mbar_wait(&bar[s], (u32)((it>>1)&1));
-        else
-        {
-            __syncwarp();
-            for(int r=0;r<rows;r++)
-            {
-                const u8 *src = p.luma+((size_t)f*p.H+(size_t)(r0+r))*p.stride;
-                u8 *dst = ring+(size_t)s*stage_bytes+(size_t)r*p.slot_bytes;
-                for(int j=lane;j<p.W;j+=32) dst[j] = __ldg(src+j);
-            }
-            __syncwarp();
-        }
+        const u8 *stage = rb.acquire(t);
+        const u8 *row = stage+(size_t)lane*p.slot_bytes;
         // which coordinates this line is read with: the frame's own without the duplicate-line check; with it only the left
         // and middle part of the frame's first line (its forced-bad middle part already presets the history median)
         const bool own = (!p.line_dup)||(frow==0);
@@ -254,8 +199,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(cons
             else bwb = bwc = bw0;
             if(lane==0) p.frame_bw[f] = bwc&0xFFFFu;
         }
-        __syncwarp();
-        if(p.use_tma&&(it+BULK_STAGES<n_items)) issue(it+BULK_STAGES);
+        rb.release(it);                                         // after the black/white pass: it reads staged rows 0, 2 and 3
         const u32 bw = (!p.line_dup||(frow==0)) ? bw0 : (((frow&1)&&(frow>=3)) ? bwc : bwb);
         const u32 rec5 = (u32)ref|((bw&0xFFFFu)<<8);
         bool line_ok = true;
@@ -309,7 +253,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(cons
             const u32 bad = __ballot_sync(0xFFFFFFFFu, active&&(!line_ok));
             if(bad) frame_bad = true;
         }
-        if(b==nbatch-1)
+        if(b==rb.nbatch-1)
         {
             if(lane==0) p.clean[f] = frame_bad ? 0 : 1;
             frame_bad = false;

@@ -5,7 +5,7 @@
 //                         one grid point per thread.
 //   pcm1_preset_kernel  : median of the four results -> per-frame presets (reference level, data coordinates).
 //   pcm1_bulk_kernel    : the HBM-bound pass.  One warp per frame, one lane per video line, 32 rows per step through a
-//                         per-warp two-stage ring of 1-D bulk copies (same transport as stc007_bulk_kernel).  Decodes
+//                         per-warp staging ring of bulk_ring.cuh, as in stc007_bulk_kernel.  Decodes
 //                         every line with the frame's presets (STG_INPUT_ALL -> first readPCMdata candidate), finds the
 //                         frame's black/white levels from the first non-header line the way the reference's first line
 //                         of the frame does, applies the per-field rules of a valid line and flags the frame clean.
@@ -15,6 +15,7 @@
 //                         are hints (re-made in the kernel when the chain holds other presets), hinted lines in the
 //                         chain's steady state are finished one per thread, lines without a valid hint get the whole block.
 #pragma once
+#include "bulk_ring.cuh"
 #include "pcm1_chain.cuh"
 #include "stc007_bulk.cuh"
 
@@ -59,19 +60,19 @@ __global__ void pcm1_preset_kernel(const P1Preset *scan, int n_frames, int H, in
     presets[f] = ps;
 }
 
-struct P1BulkParams
+struct P1BulkParams                 // pcm1_bulk_kernel and pcm16x0_bulk_kernel
 {
     const u8 *luma; int H, W; size_t stride;
     int n_frames;
     const P1Preset *presets;
     int line_dup, mode;
-    sdv_line_rec *recs; sdv_line_aux *aux;
-    u8 *clean;                      // [n_frames]: 1 = every line of the frame was taken by this kernel
-    u32 *frame_bw;                  // [n_frames]: black | white<<8 the frame's lines were given
+    sdv_line_rec *recs; sdv_line_aux *aux;     // PCM-16x0: three sub-line records per line
+    u8 *clean;                      // [n_frames]: 1 = every line of the frame was taken by the kernel
+    u32 *frame_bw;                  // [n_frames]: black | white<<8 the frame's (PCM-16x0: last) lines were given
     int use_tma, warps; u32 slot_bytes;
 };
 
-enum { P1_BULK_HEADER = 128+512+BULK_MAX_WARPS*1024 };     // barriers, CRC byte table, one histogram per warp
+enum { P1_BULK_HEADER = BULK_BAR_BYTES+512+BULK_MAX_WARPS*1024 };     // barriers, CRC byte table, one histogram per warp
 
 // Black/white levels of one staged row (findPCM1BW + findBlackWhite tail), by one warp.
 __device__ __forceinline__ u32 p1_warp_black_white(const u8 *row, int W, u32 *hist, int lane)
@@ -95,45 +96,17 @@ __device__ __forceinline__ u32 p1_warp_black_white(const u8 *row, int W, u32 *hi
 __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm1_bulk_kernel(const __grid_constant__ P1BulkParams p)
 {
     extern __shared__ __align__(128) u8 dsm[];
-    u64 *bars = (u64 *)dsm;
-    u16 *crc_tab = (u16 *)(dsm+128);                            // CRC-16 CCITT byte table
+    u16 *crc_tab = (u16 *)(dsm+BULK_BAR_BYTES);                 // CRC-16 CCITT byte table
     const int warp = threadIdx.x>>5, lane = threadIdx.x&31;
-    u32 *hist = (u32 *)(dsm+128+512)+warp*256;
-    const u32 stage_bytes = BULK_ROWS*p.slot_bytes;
-    u8 *ring = dsm+P1_BULK_HEADER+(size_t)warp*BULK_STAGES*stage_bytes;
-    u64 *bar = bars+warp*BULK_STAGES;
+    u32 *hist = (u32 *)(dsm+BULK_BAR_BYTES+512)+warp*256;
     for(int i=threadIdx.x;i<256;i+=blockDim.x) crc_tab[i] = c_crc8[i];
-    if(p.use_tma&&(lane==0))
-    {
-        for(int s=0;s<BULK_STAGES;s++) mbar_init(&bar[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    BulkRing rb(dsm, P1_BULK_HEADER, p.luma, p.H, p.W, p.stride, 0, p.n_frames, p.use_tma, p.warps, p.slot_bytes);
     __syncthreads();
+    rb.prime();
 
     const int hf = p.H/2;
-    const int nbatch = (p.H+BULK_ROWS-1)/BULK_ROWS;
-    const long long n_units = p.n_frames;
-    const long long gw = (long long)blockIdx.x*p.warps+warp, gstride = (long long)gridDim.x*p.warps;
-    const long long my_units = (gw<n_units) ? ((n_units-gw+gstride-1)/gstride) : 0;
-    const long long n_items = my_units*nbatch;
     const int fld = lane&1;
     const int pixel_stop = p.W-1;
-
-    auto issue = [&](long long it)
-    {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int r0 = (int)(it%nbatch)*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int s = (int)(it&1);
-        if(lane==0)
-        {
-            const u32 bytes = (u32)rows*(u32)p.stride;
-            mbar_expect_tx(&bar[s], bytes);
-            bulk_g2s(smem_u32(ring)+(u32)s*stage_bytes, p.luma+((size_t)u*p.H+(size_t)r0)*p.stride, bytes, &bar[s]);
-        }
-        __syncwarp();
-    };
-    if(p.use_tma) { if(n_items>0) issue(0); if(n_items>1) issue(1); }
 
     u32 c01 = 0, c23 = 0, c45 = 0;              // words of this field's last line in the previous step (duplicate check)
     bool c_hdr = false;
@@ -142,17 +115,12 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm1_bulk_kernel(const _
     int ref = 128; u32 psm = INT_CALC_MULT, half = INT_CALC_MULT/2; int ofs = 0;
     u32 rec5 = 0, rec6 = 0, picked = 0;
 
-    for(long long it=0;it<n_items;it++)
+    for(long long it=0;it<rb.n_items;it++)
     {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int b = (int)(it%nbatch), r0 = b*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int f = (int)u;
-        const int s = (int)(it&1);
+        const BulkItem t = rb.item(it);
+        const int f = t.f, b = t.b, r0 = t.r0, rows = t.rows;
         const int k = (r0>>1)+(lane>>1);
         const bool active = lane<rows;
-        const u8 *stage = ring+(size_t)s*stage_bytes;
-        const u8 *row = stage+(size_t)lane*p.slot_bytes;
         if(b==0)
         {   // frame presets from the prescan
             const P1Preset ps = p.presets[f];
@@ -170,18 +138,8 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm1_bulk_kernel(const _
             picked = (u32)t.picked_left|((u32)t.picked_right<<4);
             c01 = c23 = c45 = 0; c_hdr = false;
         }
-        if(p.use_tma) mbar_wait(&bar[s], (u32)((it>>1)&1));
-        else
-        {
-            __syncwarp();
-            for(int r=0;r<rows;r++)
-            {
-                const u8 *src = p.luma+((size_t)f*p.H+(size_t)(r0+r))*p.stride;
-                u8 *dst = ring+(size_t)s*stage_bytes+(size_t)r*p.slot_bytes;
-                for(int j=lane;j<p.W;j+=32) dst[j] = __ldg(src+j);
-            }
-            __syncwarp();
-        }
+        const u8 *stage = rb.acquire(t);
+        const u8 *row = stage+(size_t)lane*p.slot_bytes;
         // ---- 94 bit cells of this lane's row
         u32 g[4], ge[4];
         g[3] = 0; ge[3] = 0;
@@ -242,8 +200,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm1_bulk_kernel(const _
             rec5 = (u32)ref|((bw&0xFFFFu)<<8);
             if(lane==0) p.frame_bw[f] = bw&0xFFFFu;
         }
-        __syncwarp();
-        if(p.use_tma&&(it+BULK_STAGES<n_items)) issue(it+BULK_STAGES);
+        rb.release(it);                                         // after the black/white pass: it reads staged rows 0 and 2
         {
             const u32 bad = __ballot_sync(0xFFFFFFFFu, active&&((!crc_ok)||(is_hdr&&(k!=0))));
             if(bad) frame_bad = true;
@@ -286,7 +243,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm1_bulk_kernel(const _
             dst[1] = make_uint4(flags<<16, r5, r6, r7);
             if(p.aux) *(uint4 *)(p.aux+ridx) = make_uint4(is_hdr ? 0u : ((u32)ref|((u32)ref<<8)), 0u, 0u, 0u);
         }
-        if(b==nbatch-1)
+        if(b==rb.nbatch-1)
         {
             if(lane==0) p.clean[f] = frame_bad ? 0 : 1;
             frame_bad = false;

@@ -1079,50 +1079,24 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     pcm1_preset_kernel<<<(n_frames+255)/256, 256, 0, st>>>(h->p1_scan, n_frames, H, cfg->mode, h->p1_presets);
     h->stats.kernel_launches++;
     // bulk pass (only meaningful with per-frame presets, i.e. when the prescan runs)
-    const u32 copy_bytes = (u32)((W+15)&~15);
-    int use_tma = (((size_t)stride%16)==0)&&((((uintptr_t)luma_dev)%16)==0);
-    u32 slot_bytes = use_tma ? (u32)stride : (((copy_bytes/16)&1) ? copy_bytes : (copy_bytes+16));
-    int bulk_warps = (int)((size_t)(227*1024-P1_BULK_HEADER)/((size_t)BULK_STAGES*BULK_ROWS*slot_bytes));
-    if((bulk_warps<1)&&use_tma)
-    {
-        use_tma = 0; slot_bytes = ((copy_bytes/16)&1) ? copy_bytes : (copy_bytes+16);
-        bulk_warps = (int)((size_t)(227*1024-P1_BULK_HEADER)/((size_t)BULK_STAGES*BULK_ROWS*slot_bytes));
-    }
-    if(bulk_warps>BULK_MAX_WARPS) bulk_warps = BULK_MAX_WARPS;
+    const BulkPlan bulk = bulk_plan(W, stride, luma_dev, P1_BULK_HEADER);
     // the bulk pass knows the first-line rule of the duplicate-line check at its default only (en_first_line_dup): with the switch
     // off every frame goes through the chain kernel
-    const bool use_bulk = prescan&&(bulk_warps>=1)&&(H>=2*BULK_ROWS)&&p1_prescan_runs(H, false, cfg->mode)
+    const bool use_bulk = prescan&&(bulk.warps>=1)&&(H>=2*BULK_ROWS)&&p1_prescan_runs(H, false, cfg->mode)
                           &&(h->fine.en_first_line_dup||!cfg->check_line_dup);
-    if(use_bulk&&x0)
-    {
-        X0BulkParams bp;
-        bp.luma = luma_dev; bp.H = H; bp.W = W; bp.stride = (size_t)stride; bp.n_frames = n_frames;
-        bp.presets = h->p1_presets; bp.line_dup = cfg->check_line_dup ? 1 : 0; bp.mode = cfg->mode;
-        bp.recs = recs_dev; bp.aux = aux_dev; bp.clean = h->p1_clean; bp.frame_bw = h->p1_bw;
-        bp.use_tma = use_tma; bp.warps = bulk_warps; bp.slot_bytes = slot_bytes;
-        int grid = (n_frames+bulk_warps-1)/bulk_warps;
-        if(grid>h->num_sms) grid = h->num_sms;
-        const size_t smem = P1_BULK_HEADER+(size_t)bulk_warps*BULK_STAGES*BULK_ROWS*slot_bytes;
-        timing_flush(h, 0);
-        cudaEventRecord(h->ev[0], st);
-        pcm16x0_bulk_kernel<<<grid, bulk_warps*32, smem, st>>>(bp);
-        cudaEventRecord(h->ev[1], st);
-        h->ev_set[0] = 1; h->ev_units[0] = (uint64_t)n_frames*(uint64_t)H;
-        h->stats.kernel_launches++;
-    }
-    else if(use_bulk)
+    if(use_bulk)
     {
         P1BulkParams bp;
         bp.luma = luma_dev; bp.H = H; bp.W = W; bp.stride = (size_t)stride; bp.n_frames = n_frames;
         bp.presets = h->p1_presets; bp.line_dup = cfg->check_line_dup ? 1 : 0; bp.mode = cfg->mode;
         bp.recs = recs_dev; bp.aux = aux_dev; bp.clean = h->p1_clean; bp.frame_bw = h->p1_bw;
-        bp.use_tma = use_tma; bp.warps = bulk_warps; bp.slot_bytes = slot_bytes;
-        int grid = (n_frames+bulk_warps-1)/bulk_warps;
+        bp.use_tma = bulk.use_tma; bp.warps = bulk.warps; bp.slot_bytes = bulk.slot_bytes;
+        int grid = (n_frames+bulk.warps-1)/bulk.warps;
         if(grid>h->num_sms) grid = h->num_sms;
-        const size_t smem = P1_BULK_HEADER+(size_t)bulk_warps*BULK_STAGES*BULK_ROWS*slot_bytes;
         timing_flush(h, 0);
         cudaEventRecord(h->ev[0], st);
-        pcm1_bulk_kernel<<<grid, bulk_warps*32, smem, st>>>(bp);
+        if(x0) pcm16x0_bulk_kernel<<<grid, bulk.warps*32, bulk.smem, st>>>(bp);
+        else pcm1_bulk_kernel<<<grid, bulk.warps*32, bulk.smem, st>>>(bp);
         cudaEventRecord(h->ev[1], st);
         h->ev_set[0] = 1; h->ev_units[0] = (uint64_t)n_frames*(uint64_t)H;
         h->stats.kernel_launches++;
@@ -1271,22 +1245,8 @@ static int decode_frames_impl(sdv_handle *h, const sdv_bin_config *cfg, const ui
     { int rc = ensure(h, (void **)&h->clean, &h->clean_cap, 2*(size_t)n_frames+16); if(rc) return rc; }
 
 
-    // bulk kernel launch configuration
-    // Rows with a 16-byte aligned pitch are bulk-copied 32 at a time (they are contiguous): the shared-memory row pitch
-    // is then the memory pitch.  Otherwise rows are copied with plain loads into slots of an odd number of 16-byte units
-    // (fewest bank conflicts between the 32 rows a warp reads together).
-    const u32 copy_bytes = (u32)((W+15)&~15);
-    int use_tma = (((size_t)stride%16)==0)&&((((uintptr_t)luma_dev)%16)==0);
-    u32 slot_bytes = use_tma ? (u32)stride : (((copy_bytes/16)&1) ? copy_bytes : (copy_bytes+16));
-    int bulk_warps = (int)((size_t)(227*1024-BULK_SMEM_HEADER)/((size_t)BULK_STAGES*BULK_ROWS*slot_bytes));
-    if((bulk_warps<1)&&use_tma)
-    {   // very wide pitch: fall back to the compact layout
-        use_tma = 0; slot_bytes = ((copy_bytes/16)&1) ? copy_bytes : (copy_bytes+16);
-        bulk_warps = (int)((size_t)(227*1024-BULK_SMEM_HEADER)/((size_t)BULK_STAGES*BULK_ROWS*slot_bytes));
-    }
-    if(bulk_warps>BULK_MAX_WARPS) bulk_warps = BULK_MAX_WARPS;
-    if(bulk_warps<1) return fail(h, SDV_ERR_ARG, "line too wide for the bulk kernel", cudaSuccess);
-    const size_t bulk_smem = BULK_SMEM_HEADER+(size_t)bulk_warps*BULK_STAGES*BULK_ROWS*slot_bytes;
+    const BulkPlan bulk = bulk_plan(W, stride, luma_dev, BULK_SMEM_HEADER);
+    if(bulk.warps<1) return fail(h, SDV_ERR_ARG, "line too wide for the bulk kernel", cudaSuccess);
 
     // Segment mode: the tape is decoded as [chain_segments] independent files, one chain per thread block, all in
     // one launch.  For tapes whose lines keep failing the preset decode (every frame would go through the single
@@ -1354,20 +1314,19 @@ static int decode_frames_impl(sdv_handle *h, const sdv_bin_config *cfg, const ui
         bp.f0 = f_from; bp.n_frames = n_frames-f_from;
         bp.ref = b.def_ref; bp.black = b.def_black; bp.white = b.def_white; bp.line_dup = (u8)dup_flags; bp.coords = b.def_coord;
         bp.recs = recs_dev; bp.aux = aux_dev; bp.clean = h->clean; bp.first_unclean = first_unclean_dev;
-        bp.use_tma = use_tma; bp.copy_bytes = copy_bytes; bp.slot_bytes = slot_bytes; bp.warps = bulk_warps;
+        bp.use_tma = bulk.use_tma; bp.slot_bytes = bulk.slot_bytes;
         { const Ppb ppb = make_ppb(b.def_coord); for(int i=0;i<BITS_PCM_DATA;i++) bp.pos[i] = (u32)pixel_of_bit(ppb, i, 0, W-1); }
         const long long units = (long long)(n_frames-f_from);      // frames
         const bool fuse = fuse_req&&(fuse_launches==0);
-        int warps = bulk_warps; size_t smem = bulk_smem;
+        BulkPlan pl = bulk;
         if(fuse)
-        {   // room for the line words of one frame per warp
-            warps = (int)((size_t)(227*1024-BULK_SMEM_HEADER)/((size_t)BULK_STAGES*BULK_ROWS*slot_bytes+BULK_FUSE_BYTES));
-            if(warps>BULK_MAX_WARPS) warps = BULK_MAX_WARPS;
-            if(warps<1) { fuse_ok = false; warps = bulk_warps; }
-            else smem = BULK_SMEM_HEADER+(size_t)warps*((size_t)BULK_STAGES*BULK_ROWS*slot_bytes+BULK_FUSE_BYTES);
+        {   // the same slots, with room for the line words of one frame per warp
+            const BulkPlan fp = bulk_plan_warps(bulk, BULK_SMEM_HEADER, BULK_FUSE_BYTES);
+            if(fp.warps<1) fuse_ok = false;
+            else pl = fp;
         }
         const bool fuse_now = fuse&&fuse_ok;
-        bp.warps = warps;
+        bp.warps = pl.warps;
         bp.samples = NULL; bp.sflags = NULL; bp.broken_bits = NULL; bp.broken_sum = NULL; bp.block0 = 0; bp.lpf = 0;
         if(fuse_now)
         {
@@ -1379,14 +1338,14 @@ static int decode_frames_impl(sdv_handle *h, const sdv_bin_config *cfg, const ui
         }
         else if(fuse_req) fuse_ok = false;                          // a second bulk launch: its frames are not fused
         fuse_launches++;
-        int grid = (int)((units+warps-1)/warps);
+        int grid = (int)((units+pl.warps-1)/pl.warps);
         // the fused pass carries ~10 % more instructions per line: every SM but the one the first-frame chain block needs
         const int max_blocks = (fuse_now&&(bulk_blocks_env<=0)&&(h->num_sms>8)) ? (h->num_sms-1) : bulk_blocks;
         if(grid>max_blocks) grid = max_blocks;
         timing_flush(h, 0);
         cudaEventRecord(h->ev[0], bst);
-        if(fuse_now) stc007_bulk_kernel<true><<<grid, warps*32, smem, bst>>>(bp);
-        else stc007_bulk_kernel<false><<<grid, warps*32, smem, bst>>>(bp);
+        if(fuse_now) stc007_bulk_kernel<true><<<grid, pl.warps*32, pl.smem, bst>>>(bp);
+        else stc007_bulk_kernel<false><<<grid, pl.warps*32, pl.smem, bst>>>(bp);
         cudaEventRecord(h->ev[1], bst);
         h->ev_set[0] = 1; h->ev_units[0] = (uint64_t)(n_frames-f_from)*(uint64_t)H;
         h->stats.kernel_launches++;

@@ -6,14 +6,14 @@
 // VideoToDigital applies to a valid line (first PCM line of a field, duplicate line; videotodigital.cpp:1159-1278).
 // A field in which every line decodes this way is flagged clean; everything else is redone by stc007_chain_kernel.
 //
-// How: one LANE per video line, 32 lines of one field per warp step.  The 32 rows arrive in shared memory through a
-// per-warp double-buffered ring of 1-D bulk TMA copies (cp.async.bulk.shared.global + mbarrier complete_tx), one copy
-// per lane.  Each lane walks the 128 bit-cell centres of its row: one byte load per cell (the cell positions are
+// How: one LANE per video line, 32 consecutive rows of a frame per warp step, staged in shared memory by the per-warp
+// ring of bulk_ring.cuh (one 1-D bulk copy per step).  Each lane walks the 128 bit-cell centres of its row: one byte load per cell (the cell positions are
 // launch constants read from the kernel parameter bank), and two funnel-shift registers accumulate "pixel > ref" and
 // "pixel >= ref" MSB-first, which is already the bit order of the PCM words.  Cells sitting exactly on the reference
 // level keep the previous bit (the reference's level hysteresis at depth 0): resolved per lane as a 128-bit carry
 // chain.  CRCC by a 256-entry table in shared memory, 14 steps.  Two 16-byte stores per lane write the line record.
 #pragma once
+#include "bulk_ring.cuh"
 #include "stc007_chain.cuh"
 #include "stc007_deint.cuh"
 
@@ -21,32 +21,7 @@ namespace sdv {
 
 __constant__ u16 c_crc8[3*256];     // [0..255]: CRC-16 CCITT byte table (CRC, init 0, of the byte x);
                                     // [256..511] / [512..767]: the CRC state x / x<<8 advanced over 7 zero bytes
-enum { BULK_SMEM_HEADER = 128+3*512 };
-
-__device__ __forceinline__ u32 smem_u32(const void *p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64 *bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(u64 *bar, u32 bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity)
-{
-    u32 done;
-    do
-    {
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    }
-    while(!done);
-}
-__device__ __forceinline__ void bulk_g2s(u32 dst_smem, const void *src, u32 bytes, u64 *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(dst_smem), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
+enum { BULK_SMEM_HEADER = BULK_BAR_BYTES+3*512 };
 
 struct BulkParams
 {
@@ -56,7 +31,7 @@ struct BulkParams
     sdv_line_rec *recs; sdv_line_aux *aux;
     u8 *clean;                      // [2*total frames] per field: 1 = every line of the field was taken by this kernel
     int *first_unclean;             // atomicMin of the frames with a field that is not clean
-    int use_tma, warps; u32 copy_bytes, slot_bytes;
+    int use_tma, warps; u32 slot_bytes;
     u32 pos[BITS_PCM_DATA];         // pixel of each bit cell centre (PCMLine::getVideoPixeBylCalc, pcmline.cpp:249-311)
     // Fused deinterleave (stc007_bulk_kernel<true>): the warp that decoded a frame keeps its line words in shared memory and
     // finishes, when the frame is complete, every data block whose eight lines lie inside the frame (the first 2*lpf - 112 of the
@@ -115,55 +90,25 @@ __device__ __forceinline__ bool packed_control_block(u32 w01, u32 w23, u32 w45, 
     return (w01==0x0CCC3333u)&&(w23==0x0CCC3333u)&&((w45&0xFFFFu)==0)&&(((w67>>16)&0x0FF0u)==0);
 }
 
-enum { BULK_MAX_WARPS = 4, BULK_STAGES = 2, BULK_ROWS = 32 };
-
 template<bool FUSE>
 __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) stc007_bulk_kernel(const __grid_constant__ BulkParams p)
 {
     extern __shared__ __align__(128) u8 dsm[];
-    u64 *bars = (u64 *)dsm;                                     // [warps][BULK_STAGES]
-    u16 *crc_tab = (u16 *)(dsm+128);                            // [3][256]: byte table, 7-byte advance of the low / high CRC byte
+    u16 *crc_tab = (u16 *)(dsm+BULK_BAR_BYTES);                 // [3][256]: byte table, 7-byte advance of the low / high CRC byte
     const int warp = threadIdx.x>>5, lane = threadIdx.x&31;
-    const u32 stage_bytes = BULK_ROWS*p.slot_bytes;
-    u8 *ring = dsm+BULK_SMEM_HEADER+(size_t)warp*BULK_STAGES*stage_bytes;
-    u64 *bar = bars+warp*BULK_STAGES;
     // fused deinterleave: this warp's line words of the current frame, word-major per field, and a valid flag per line
-    u16 *fw = (u16 *)(dsm+BULK_SMEM_HEADER+(size_t)p.warps*BULK_STAGES*stage_bytes+(size_t)warp*BULK_FUSE_BYTES);
+    u16 *fw = (u16 *)(dsm+BULK_SMEM_HEADER+(size_t)p.warps*BULK_STAGES*BULK_ROWS*p.slot_bytes+(size_t)warp*BULK_FUSE_BYTES);
     u8 *fok = (u8 *)(fw+2*8*BULK_FUSE_HF);
     for(int i=threadIdx.x;i<3*256;i+=blockDim.x) crc_tab[i] = c_crc8[i];
-    if(p.use_tma&&(lane==0))
-    {
-        for(int s=0;s<BULK_STAGES;s++) mbar_init(&bar[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    BulkRing rb(dsm, BULK_SMEM_HEADER, p.luma, p.H, p.W, p.stride, p.f0, p.n_frames, p.use_tma, p.warps, p.slot_bytes);
     __syncthreads();
+    rb.prime();
 
-    // Work unit = one frame: BULK_ROWS consecutive rows of the frame per step (rows alternate between the two fields:
-    // lane l holds field l&1, line (l>>1) of the step), so that one bulk copy brings the whole step.
+    // A step holds BULK_ROWS consecutive rows of the frame: rows alternate between the two fields, lane l holds field l&1,
+    // line (l>>1) of the step.
     const int hf = p.H/2;
-    const int nbatch = (p.H+BULK_ROWS-1)/BULK_ROWS;
-    const long long n_units = p.n_frames;
-    const long long gw = (long long)blockIdx.x*p.warps+warp, gstride = (long long)gridDim.x*p.warps;
-    const long long my_units = (gw<n_units) ? ((n_units-gw+gstride-1)/gstride) : 0;
-    const long long n_items = my_units*nbatch;                  // item = one step of BULK_ROWS rows
     const int ref = p.ref;
     const int fld = lane&1;
-
-    auto issue = [&](long long it)
-    {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int r0 = (int)(it%nbatch)*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int s = (int)(it&1);
-        if(lane==0)
-        {
-            const u32 bytes = (u32)rows*(u32)p.stride;          // the rows are contiguous in memory: one copy
-            mbar_expect_tx(&bar[s], bytes);
-            bulk_g2s(smem_u32(ring)+(u32)s*stage_bytes, p.luma+((size_t)(p.f0+u)*p.H+(size_t)r0)*p.stride, bytes, &bar[s]);
-        }
-        __syncwarp();
-    };
-    if(p.use_tma) { if(n_items>0) issue(0); if(n_items>1) issue(1); }
 
     u32 c01 = 0, c23 = 0, c45 = 0, c67 = 0;     // words of this field's last line in the previous step (duplicate check)
     bool c_cb = false;
@@ -171,28 +116,13 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) stc007_bulk_kernel(const
     const u32 rec5 = (u32)p.ref|((u32)p.black<<8)|((u32)p.white<<16);                // ref, black, white, hyst = 0
     const u32 rec6 = (u32)(u16)p.coords.start|((u32)(u16)p.coords.stop<<16);
 
-    for(long long it=0;it<n_items;it++)
+    for(long long it=0;it<rb.n_items;it++)
     {
-        const long long u = gw+(it/nbatch)*gstride;
-        const int b = (int)(it%nbatch), r0 = b*BULK_ROWS;
-        const int rows = (p.H-r0<BULK_ROWS) ? (p.H-r0) : BULK_ROWS;
-        const int f = p.f0+(int)u;
-        const int s = (int)(it&1);
+        const BulkItem t = rb.item(it);
+        const int f = t.f, b = t.b, r0 = t.r0, rows = t.rows;
         const int k = (r0>>1)+(lane>>1);                        // line of the field
         const bool active = lane<rows;
-        const u8 *row = ring+(size_t)s*stage_bytes+(size_t)lane*p.slot_bytes;
-        if(p.use_tma) mbar_wait(&bar[s], (u32)((it>>1)&1));
-        else
-        {   // rows that cannot be bulk-copied (unaligned stride): plain loads into the same layout
-            __syncwarp();
-            for(int r=0;r<rows;r++)
-            {
-                const u8 *src = p.luma+((size_t)f*p.H+(size_t)(r0+r))*p.stride;
-                u8 *dst = ring+(size_t)s*stage_bytes+(size_t)r*p.slot_bytes;
-                for(int j=lane;j<p.W;j+=32) dst[j] = __ldg(src+j);
-            }
-            __syncwarp();
-        }
+        const u8 *row = rb.acquire(t)+(size_t)lane*p.slot_bytes;
         // ---- 128 bit cells of this lane's row
         u32 g[4], ge[4];
 #pragma unroll
@@ -208,8 +138,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) stc007_bulk_kernel(const
             }
             g[w] = a; ge[w] = c;
         }
-        __syncwarp();
-        if(p.use_tma&&(it+BULK_STAGES<n_items)) issue(it+BULK_STAGES);      // the slot is free again
+        rb.release(it);
         const bool any_eq = ((ge[0]^g[0])|(ge[1]^g[1])|(ge[2]^g[2])|(ge[3]^g[3]))!=0;
         if(__any_sync(0xFFFFFFFFu, any_eq)) resolve_equal_cells(g, ge);
         // ---- words and CRCC (two independent table chains over the two halves of the 14-byte message)
@@ -297,7 +226,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) stc007_bulk_kernel(const
                 d[4*BULK_FUSE_HF] = (u16)w45; d[5*BULK_FUSE_HF] = (u16)(w45>>16); d[6*BULK_FUSE_HF] = (u16)w67; d[7*BULK_FUSE_HF] = (u16)(w67>>16);
                 fok[fld*BULK_FUSE_HF+k] = ((flags&SDV_LF_CRC_OK)&&!is_cb) ? 1 : 0;      // line_rec_ok: a service line gives no trusted words
             }
-            if(b==nbatch-1)
+            if(b==rb.nbatch-1)
             {   // every block of this frame whose lines all lie inside it: assembled line a = field 0 lines, lpf - hf empty lines,
                 // field 1 lines, empty lines; block a takes word j of line a + 16 j
                 __syncwarp();
@@ -337,7 +266,7 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) stc007_bulk_kernel(const
                 __syncwarp();
             }
         }
-        if(b==nbatch-1)
+        if(b==rb.nbatch-1)
         {   // frame done
             if(lane<2) p.clean[2*(size_t)f+lane] = ((frame_bad>>lane)&1u) ? 0 : 1;
             if((lane==0)&&frame_bad) atomicMin(p.first_unclean, f);
