@@ -103,7 +103,7 @@ class BinStats(C.Structure):
 
 class Pcm16x0Config(C.Structure):
     _fields_ = [("ignore_crc", C.c_uint8), ("force_check", C.c_uint8), ("p_corr", C.c_uint8), ("ei_format", C.c_uint8),
-                ("reserved", C.c_uint8 * 4)]
+                ("continue_file", C.c_uint8), ("reserved", C.c_uint8 * 3)]
 
 
 class Pcm1StitchConfig(C.Structure):

@@ -15,6 +15,7 @@ struct X0ChainCtx
     Coord long_valid[COORD_LONG_HISTORY];
     int n_last, n_long;
     Coord frame_avg;
+    P1Preset run_g;                         // presets of the file's first frame: the running pair G of the bulk pass
     int n_fv, n_fi;
     int good_in_field, pcm_in_field, line_in_field;
     Coord frame_valid[SDV_MAX_H*3];

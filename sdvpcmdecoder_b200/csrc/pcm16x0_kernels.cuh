@@ -7,7 +7,8 @@
 //                            With the duplicate-line check on, the reference decodes only the first line of a frame with
 //                            the frame's prescan coordinates: that line is forced bad, its right part then presets the
 //                            median of the coordinate history (videotodigital.cpp:1427-1516) and every later line follows
-//                            it -- so the pass runs with one running coordinate pair G (the first frame's) plus the
+//                            it -- so the pass runs with one running coordinate pair G (the file's first frame's; a call
+//                            that continues the file reads it from the chain context) plus the
 //                            per-frame reference level, and with three black/white measurements per frame (first line,
 //                            second line of either field).  Frames decoded completely this way are flagged clean.
 //   pcm16x0_chain_kernel   : walks the frames in order; skips runs of clean frames while the chain state is the steady one
@@ -19,14 +20,14 @@
 
 namespace sdv {
 
-__global__ void __launch_bounds__(P1S_THREADS, 5) pcm16x0_prescan_kernel(const u8 *luma, int H, int W, size_t stride, int n_frames, int mode, P1Preset *scan)
+__global__ void __launch_bounds__(P1S_THREADS, 5) pcm16x0_prescan_kernel(const u8 *luma, int H, int W, size_t stride, int n_frames, int mode, int opens, P1Preset *scan)
 {
     __shared__ X0Work w;
     __shared__ __align__(16) u8 px[SDV_MAX_W];
     const int f = blockIdx.x/P1_COORD_CHECK_LINES, idx = blockIdx.x%P1_COORD_CHECK_LINES;
     if(f>=n_frames) return;
     P1Preset r; r.valid = 0; r.ref = 0; r.coords = coord_none(); r.pad[0] = r.pad[1] = 0;
-    const int row = p1_prescan_row(H, f==0, idx);
+    const int row = p1_prescan_row(H, opens&&(f==0), idx);
     if(row<0) { if(threadIdx.x==0) scan[blockIdx.x] = r; return; }
     const u8 *src = luma+((size_t)f*H+(size_t)row)*stride;
     for(int i=threadIdx.x;i<W;i+=blockDim.x) px[i] = __ldg(src+i);
@@ -108,8 +109,8 @@ __global__ void __launch_bounds__(BULK_MAX_WARPS*32, 1) pcm16x0_bulk_kernel(cons
     const int fld = lane&1;
     const int pixel_stop = p.W-1;
 
-    // the running coordinates of the tape (duplicate-line check on): those of the first frame
-    const P1Preset ps0 = p.presets[0];
+    // the running coordinates of the tape (duplicate-line check on): those of the file's first frame
+    const P1Preset ps0 = *p.run_g;
     const bool have_g = ps0.valid&&coord_valid(ps0.coords);
     Coord gc = ps0.coords; if(!have_g) { gc.start = 0; gc.stop = (i16)(p.W-1); }
     const Ppb gpp = x0_make_ppb(gc);
@@ -268,6 +269,7 @@ struct X0ChainParams
 {
     const u8 *luma; int H, W; size_t stride; int n_frames;
     int mode, line_dup, use_bulk;
+    int cont;                       // the call continues the file: the chain starts from *ctx instead of a reset
     const P1Preset *scan; const P1Preset *presets; const u8 *clean; const u32 *frame_bw;
     sdv_line_rec *recs; sdv_line_aux *aux;
     X0ChainCtx *ctx;
@@ -278,7 +280,7 @@ struct X0ChainParams
 __device__ __forceinline__ u8 x0_scan_done_of(const X0ChainParams &p, int f, bool ran, int row)
 {
     u8 sd = 0;
-    if(ran) for(int idx=0;idx<P1_COORD_CHECK_LINES;idx++) if(p1_prescan_row(p.H, f==0, idx)==row) sd = p.scan[(size_t)f*P1_COORD_CHECK_LINES+idx].pad[0];
+    if(ran) for(int idx=0;idx<P1_COORD_CHECK_LINES;idx++) if(p1_prescan_row(p.H, (!p.cont)&&(f==0), idx)==row) sd = p.scan[(size_t)f*P1_COORD_CHECK_LINES+idx].pad[0];
     return sd;
 }
 // The sub-line object of a hinted sub-line (preset-only decode, first readPCMdata candidate valid).
@@ -320,9 +322,12 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm16x0_chain_kernel(X0ChainParam
     X0ChainCtx *x = (X0ChainCtx *)chain_dsm;
     const int hf = p.H/2;
     const int depth = COORD_HISTORY_DEPTH*3;
-    if(c.tid==0) { x0_chain_reset(x, p.mode, p.line_dup); p.stats[0] = p.stats[1] = p.stats[2] = p.stats[3] = 0; }
+    if(p.cont) { for(int i=c.tid;i<(int)(sizeof(X0ChainCtx)/4);i+=c.n) ((u32 *)x)[i] = ((const u32 *)p.ctx)[i]; }
+    else if(c.tid==0) { x0_chain_reset(x, p.mode, p.line_dup); x->run_g = p.presets[0]; }
+    if(c.tid==0) { p.stats[0] = p.stats[1] = p.stats[2] = p.stats[3] = 0; }
     __syncthreads();
-    const P1Preset ps0 = p.presets[0];
+    const bool opens = !p.cont;         // frame 0 carries the NEW_FILE line
+    const P1Preset ps0 = x->run_g;      // the running pair G the bulk pass decoded with
     int f = 0;
     while(f<p.n_frames)
     {
@@ -335,10 +340,11 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm16x0_chain_kernel(X0ChainParam
             if(ff<p.n_frames)
             {
                 const P1Preset ps = p.presets[ff];
-                ok = p.clean[ff]&&ps.valid&&coord_valid(ps.coords)&&p1_prescan_runs(p.H, ff==0, p.mode);
+                ok = p.clean[ff]&&ps.valid&&coord_valid(ps.coords)&&p1_prescan_runs(p.H, opens&&(ff==0), p.mode);
                 if(ok&&p.line_dup)
-                {   // steady state the bulk pass assumed: the whole coordinate history equals the running pair G
-                    if((c.tid==0)&&(ff>0))
+                {   // steady state the bulk pass assumed: the whole coordinate history equals the running pair G (only the
+                    // file's first frame is decoded with G as its own prescan coordinates)
+                    if((c.tid==0)&&((ff>0)||!opens))
                     {
                         if(x->n_last!=depth) ok = false;
                         for(int i=0;ok&&(i<x->n_last);i++) if(!coord_eq(x->last_valid[i], ps0.coords)) ok = false;
@@ -381,7 +387,7 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm16x0_chain_kernel(X0ChainParam
             }
         }
         // ---- exact sequential decode of frame f
-        const bool ran = p1_prescan_runs(p.H, f==0, p.mode);
+        const bool ran = p1_prescan_runs(p.H, opens&&(f==0), p.mode);
         if(c.tid==0) x0_chain_frame_start(x, ran, p.presets[f]);
         __syncthreads();
         for(int fld=0;fld<2;fld++)

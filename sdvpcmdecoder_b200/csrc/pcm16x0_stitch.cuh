@@ -124,10 +124,12 @@ SDV_HD u8 x0_ctrl_votes(const X0AsmScratch *s)
     if((cnt[0]>=2)&&(cnt[1]>=2)&&(cnt[3]>=2)) v |= SDV_X0I_VALID;
     return v;
 }
+enum { X0_CTRL_HISTORY = 64 };       // frames before the current one whose votes count (updateCtrlBitStats keeps 65 with it)
 // What frame f works with (f1_srate, f1_emph, f1_code at the end of fillFrameForOutput, 4711-4741): its own vote, or the
 // majority over the last 65 frames (updateCtrlBitStats + getProbable*, 4126-4348; ties and an empty history give 44056 Hz /
-// true / true -- the fall-back booleans are "bit is 1", the opposite sense of the voted ones).
-SDV_HD void x0_ctrl_effective(sdv_pcm16x0_frame_info *info, int f)
+// true / true -- the fall-back booleans are "bit is 1", the opposite sense of the voted ones).  hist: the votes of the
+// X0_CTRL_HISTORY frames before frame 0 of the call (hist[X0_CTRL_HISTORY-1] = the frame just before), NULL = none.
+SDV_HD void x0_ctrl_effective(sdv_pcm16x0_frame_info *info, int f, const u8 *hist = 0)
 {
     const u8 v = info[f].frame_votes;
     sdv_pcm16x0_frame_info o = info[f];
@@ -140,9 +142,9 @@ SDV_HD void x0_ctrl_effective(sdv_pcm16x0_frame_info *info, int f)
     else
     {
         int e_on = 0, e_off = 0, c_code = 0, c_audio = 0, r441 = 0, r440 = 0;
-        for(int g=(f>=64) ? (f-64) : 0;g<=f;g++)
+        for(int g=(hist||(f>=X0_CTRL_HISTORY)) ? (f-X0_CTRL_HISTORY) : 0;g<=f;g++)
         {
-            const u8 h = info[g].frame_votes;
+            const u8 h = (g<0) ? hist[X0_CTRL_HISTORY+g] : info[g].frame_votes;
             if(!(h&SDV_X0I_VALID)) continue;
             if(h&SDV_X0I_EMPHASIS) e_on++; else e_off++;
             if(h&SDV_X0I_CODE) c_code++; else c_audio++;
@@ -161,7 +163,8 @@ struct X0FieldGeo { i16 top_pad, cut, lines, pad; };
 
 SDV_HD void x0_stitch_frame_cta(const Cta &c, const sdv_line_rec *fr, int H, bool bff, int top_pad_odd, int top_pad_even, X0Cfg cfg,
                                 int broken_mask_dur, bool mask_seams, X0AsmScratch *s, i16 *samples, u8 *sflags,
-                                sdv_pcm16x0_frame_info *info = 0, const X0FieldGeo *geo = 0 /*[2]: odd, even field*/, bool ei = false)
+                                sdv_pcm16x0_frame_info *info = 0, const X0FieldGeo *geo = 0 /*[2]: odd, even field*/, bool ei = false,
+                                u8 *vote = 0 /*where the frame's control-bit vote is kept for the next call, may be NULL*/)
 {
     const int hf = H/2;
     const int BIG = 1<<30;
@@ -227,11 +230,12 @@ SDV_HD void x0_stitch_frame_cta(const Cta &c, const sdv_line_rec *fr, int H, boo
         for(int part=0;part<3;part++) s->sub[(size_t)i*3+part] = o[part];
     }
     c.sync();
-    if(info&&(c.tid==0))
+    if((info||vote)&&(c.tid==0))
     {
         sdv_pcm16x0_frame_info o; o.sample_rate = 0; o.emphasis = o.code = 0; o.frame_votes = x0_ctrl_votes(s);
         o.reserved[0] = o.reserved[1] = o.reserved[2] = 0;
-        *info = o;
+        if(info) *info = o;
+        if(vote) *vote = o.frame_votes;
     }
     // ---- performDeinterleave: data block q = 35*m + i from sub-lines i, i+35, i+70 of interleave block m (SI format);
     //      data block q from sub-lines q, q+490, q+980 of the frame (EI format, 5181-5186)
@@ -627,17 +631,27 @@ SDV_HD void x0_eipad_scan_cta(const Cta &c, const sdv_line_rec *fr, int H, bool 
 }
 
 #if defined(__CUDACC__)
+// The control-bit votes of the last X0_CTRL_HISTORY frames of the file as the call leaves them, into hist_out: the frames of the call,
+// in front of them the tail of hist_in (the same of the call before; NULL = the call opens the history).  Returns where frame f's
+// vote goes, NULL when it is not among the last ones.
+__device__ __forceinline__ u8 *x0_votes_carry(const Cta &c, int f, int n_frames, const u8 *hist_in, u8 *hist_out)
+{
+    if(f==0) for(int i=c.tid;i<X0_CTRL_HISTORY-n_frames;i+=c.n) hist_out[i] = hist_in ? hist_in[n_frames+i] : (u8)0;
+    return (f+X0_CTRL_HISTORY>=n_frames) ? hist_out+(X0_CTRL_HISTORY-n_frames+f) : (u8 *)0;
+}
 __global__ void __launch_bounds__(512) pcm16x0_stitch_kernel(const sdv_line_rec *recs, int n_frames, int H, int bff, int top_pad_odd,
                                                              int top_pad_even, X0Cfg cfg, int broken_mask_dur, const u8 *mask_seams,
-                                                             i16 *samples, u8 *sflags, sdv_pcm16x0_frame_info *info, int ei)
+                                                             i16 *samples, u8 *sflags, sdv_pcm16x0_frame_info *info, int ei,
+                                                             const u8 *hist_in, u8 *hist_out)
 {
     __shared__ X0AsmScratch s;
     const int f = blockIdx.x;
     if(f>=n_frames) return;
     Cta c = { (int)threadIdx.x, (int)blockDim.x };
+    u8 *vote = x0_votes_carry(c, f, n_frames, hist_in, hist_out);
     x0_stitch_frame_cta(c, recs+(size_t)f*H*3, H, bff!=0, top_pad_odd, top_pad_even, cfg, broken_mask_dur, mask_seams ? (mask_seams[f]!=0) : false, &s,
                         samples+(size_t)f*X0S_BLOCKS_FRAME*6, sflags ? sflags+(size_t)f*X0S_BLOCKS_FRAME*6 : (u8 *)0, info ? info+f : (sdv_pcm16x0_frame_info *)0,
-                        (const X0FieldGeo *)0, ei!=0);
+                        (const X0FieldGeo *)0, ei!=0, vote);
 }
 // One block per (frame, field): the padding scan of x0_sipad_scan_cta.
 __global__ void __launch_bounds__(256) pcm16x0_sipad_kernel(const sdv_line_rec *recs, int n_frames, int H, X0Cfg cfg, X0PadScan *out)
@@ -651,15 +665,16 @@ __global__ void __launch_bounds__(256) pcm16x0_sipad_kernel(const sdv_line_rec *
 // The frame stitcher with the alignment of every field given per frame (geo[2*f], geo[2*f+1]: odd, even field).
 __global__ void __launch_bounds__(512) pcm16x0_stitch_geo_kernel(const sdv_line_rec *recs, int n_frames, int H, int bff, const X0FieldGeo *geo, X0Cfg cfg,
                                                                  int broken_mask_dur, const u8 *mask_seams, i16 *samples, u8 *sflags, sdv_pcm16x0_frame_info *info,
-                                                                 int ei)
+                                                                 int ei, const u8 *hist_in, u8 *hist_out)
 {
     __shared__ X0AsmScratch s;
     const int f = blockIdx.x;
     if(f>=n_frames) return;
     Cta c = { (int)threadIdx.x, (int)blockDim.x };
+    u8 *vote = x0_votes_carry(c, f, n_frames, hist_in, hist_out);
     x0_stitch_frame_cta(c, recs+(size_t)f*H*3, H, bff!=0, 0, 0, cfg, broken_mask_dur, mask_seams ? (mask_seams[f]!=0) : false, &s,
                         samples+(size_t)f*X0S_BLOCKS_FRAME*6, sflags ? sflags+(size_t)f*X0S_BLOCKS_FRAME*6 : (u8 *)0, info ? info+f : (sdv_pcm16x0_frame_info *)0,
-                        geo+2*(size_t)f, ei!=0);
+                        geo+2*(size_t)f, ei!=0, vote);
 }
 // One block per frame: the EI padding scan of x0_eipad_scan_cta.
 __global__ void __launch_bounds__(256) pcm16x0_eipad_kernel(const sdv_line_rec *recs, int n_frames, int H, int bff, X0Cfg cfg, X0EIScan *out)
@@ -670,10 +685,10 @@ __global__ void __launch_bounds__(256) pcm16x0_eipad_kernel(const sdv_line_rec *
     Cta c = { (int)threadIdx.x, (int)blockDim.x };
     x0_eipad_scan_cta(c, recs+(size_t)f*H*3, H, bff!=0, cfg, &s, out+f);
 }
-__global__ void pcm16x0_ctrl_history_kernel(sdv_pcm16x0_frame_info *info, int n_frames)
+__global__ void pcm16x0_ctrl_history_kernel(sdv_pcm16x0_frame_info *info, int n_frames, const u8 *hist)
 {
     const int f = blockIdx.x*blockDim.x+threadIdx.x;
-    if(f<n_frames) x0_ctrl_effective(info, f);       // reads frame_votes of 65 frames, writes the other fields of its own
+    if(f<n_frames) x0_ctrl_effective(info, f, hist);     // reads frame_votes of 65 frames, writes the other fields of its own
 }
 #endif
 

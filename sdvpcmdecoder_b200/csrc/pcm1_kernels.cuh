@@ -25,14 +25,15 @@ enum { P1L_THREADS = 256, P1C_CHUNK = 256 };     // chain kernel: records staged
 enum { P1S_THREADS = 128 };                      // prescan kernels: a search is a chain of short phases, few of them wider than 64 threads -- what
                                                  // counts is how many searches an SM holds at once (8 blocks of 128 threads at 64 registers)
 
-__global__ void __launch_bounds__(P1S_THREADS, 8) pcm1_prescan_kernel(const u8 *luma, int H, int W, size_t stride, int n_frames, int mode, P1Preset *scan)
+// opens: frame 0 of the call opens the file (carries the NEW_FILE line); 0 when the call continues the previous call's file.
+__global__ void __launch_bounds__(P1S_THREADS, 8) pcm1_prescan_kernel(const u8 *luma, int H, int W, size_t stride, int n_frames, int mode, int opens, P1Preset *scan)
 {
     __shared__ P1Work w;
     __shared__ __align__(16) u8 px[SDV_MAX_W];
     const int f = blockIdx.x/P1_COORD_CHECK_LINES, idx = blockIdx.x%P1_COORD_CHECK_LINES;
     if(f>=n_frames) return;
     P1Preset r; r.valid = 0; r.ref = 0; r.coords = coord_none(); r.pad[0] = r.pad[1] = 0;
-    const int row = p1_prescan_row(H, f==0, idx);
+    const int row = p1_prescan_row(H, opens&&(f==0), idx);
     if(row<0) { if(threadIdx.x==0) scan[blockIdx.x] = r; return; }
     const u8 *src = luma+((size_t)f*H+(size_t)row)*stride;
     for(int i=threadIdx.x;i<W;i+=blockDim.x) px[i] = __ldg(src+i);
@@ -51,12 +52,12 @@ __global__ void __launch_bounds__(P1S_THREADS, 8) pcm1_prescan_kernel(const u8 *
     }
 }
 
-__global__ void pcm1_preset_kernel(const P1Preset *scan, int n_frames, int H, int mode, P1Preset *presets)
+__global__ void pcm1_preset_kernel(const P1Preset *scan, int n_frames, int H, int mode, int opens, P1Preset *presets)
 {
     const int f = blockIdx.x*blockDim.x+threadIdx.x;
     if(f>=n_frames) return;
     P1Preset ps; ps.valid = 0; ps.ref = 0; ps.coords = coord_none(); ps.pad[0] = ps.pad[1] = 0;
-    if(p1_prescan_runs(H, f==0, mode)) ps = p1_prescan_reduce(scan+(size_t)f*P1_COORD_CHECK_LINES);
+    if(p1_prescan_runs(H, opens&&(f==0), mode)) ps = p1_prescan_reduce(scan+(size_t)f*P1_COORD_CHECK_LINES);
     presets[f] = ps;
 }
 
@@ -65,6 +66,7 @@ struct P1BulkParams                 // pcm1_bulk_kernel and pcm16x0_bulk_kernel
     const u8 *luma; int H, W; size_t stride;
     int n_frames;
     const P1Preset *presets;
+    const P1Preset *run_g;          // PCM-16x0: presets of the file's first frame (the running pair G), presets[0] or the chain's copy
     int line_dup, mode;
     sdv_line_rec *recs; sdv_line_aux *aux;     // PCM-16x0: three sub-line records per line
     u8 *clean;                      // [n_frames]: 1 = every line of the frame was taken by the kernel
@@ -256,6 +258,7 @@ struct P1ChainParams
 {
     const u8 *luma; int H, W; size_t stride; int n_frames;
     int mode, line_dup, use_bulk;
+    int cont;                       // the call continues the file: the chain starts from *ctx instead of a reset
     const P1Preset *presets; const u8 *clean; const u32 *frame_bw;
     sdv_line_rec *recs; sdv_line_aux *aux;
     P1ChainCtx *ctx;
@@ -312,8 +315,11 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm1_chain_kernel(P1ChainParams p
     extern __shared__ __align__(16) u8 chain_dsm[];
     P1ChainCtx *x = (P1ChainCtx *)chain_dsm;
     const int hf = p.H/2;
-    if(c.tid==0) { p1_chain_reset(x, p.mode, p.line_dup); p.stats[0] = p.stats[1] = p.stats[2] = p.stats[3] = 0; }
+    if(p.cont) { for(int i=c.tid;i<(int)(sizeof(P1ChainCtx)/4);i+=c.n) ((u32 *)x)[i] = ((const u32 *)p.ctx)[i]; }
+    else if(c.tid==0) p1_chain_reset(x, p.mode, p.line_dup);
+    if(c.tid==0) { p.stats[0] = p.stats[1] = p.stats[2] = p.stats[3] = 0; }
     __syncthreads();
+    const bool opens = !p.cont;         // frame 0 carries the NEW_FILE line
     int f = 0;
     while(f<p.n_frames)
     {
@@ -327,9 +333,9 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm1_chain_kernel(P1ChainParams p
             if(ff<p.n_frames)
             {
                 const P1Preset ps = p.presets[ff];
-                ok = p.clean[ff]&&ps.valid&&coord_valid(ps.coords)&&p1_prescan_runs(p.H, ff==0, p.mode);
+                ok = p.clean[ff]&&ps.valid&&coord_valid(ps.coords)&&p1_prescan_runs(p.H, opens&&(ff==0), p.mode);
                 if(ok)
-                {
+                {   // thread 0 checks against the chain's history (carried over on a continuing call), the others against the frame before
                     if(c.tid==0) { for(int i=0;i<x->n_last;i++) if(!p1_within_damper(ps.coords, x->last_valid[i])) ok = false; }
                     else { const P1Preset pv = p.presets[ff-1]; ok = p1_within_damper(ps.coords, pv.coords); }
                 }
@@ -363,7 +369,7 @@ __global__ void __launch_bounds__(P1L_THREADS) pcm1_chain_kernel(P1ChainParams p
             }
         }
         // ---- exact sequential decode of frame f
-        if(c.tid==0) p1_chain_frame_start(x, p1_prescan_runs(p.H, f==0, p.mode), p.presets[f]);
+        if(c.tid==0) p1_chain_frame_start(x, p1_prescan_runs(p.H, opens&&(f==0), p.mode), p.presets[f]);
         __syncthreads();
         for(int fld=0;fld<2;fld++)
         {

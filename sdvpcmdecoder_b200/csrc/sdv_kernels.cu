@@ -908,6 +908,8 @@ struct sdv_handle
     u32 *p1_bw; size_t p1_bw_cap;
     P1ChainCtx *p1_ctx;
     X0ChainCtx *x0_ctx;
+    int pcm_open, pcm_type, pcm_H, pcm_W, pcm_mode;    // p1_ctx / x0_ctx hold the chain state at the end of the last PCM-1 / PCM-16x0 decode
+    u8 *x0_votes; int x0_votes_cur, x0_votes_open;     // control-bit votes of the last X0_CTRL_HISTORY frames of the PCM-16x0 stitch calls (two buffers)
     unsigned long long *p1_stats_dev, *p1_stats_host;
     sdv_pcm1_subline *p1_sub; size_t p1_sub_cap;  // assembled fields (sdv_pcm1_frames_to_samples)
     char err[256];
@@ -999,6 +1001,7 @@ int sdv_create(sdv_handle **out, int cuda_device)
     if(e==cudaSuccess) e = cudaFuncSetAttribute(pcm1_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227*1024);
     if(e==cudaSuccess) e = cudaMalloc(&h->p1_ctx, sizeof(P1ChainCtx));
     if(e==cudaSuccess) e = cudaMalloc(&h->x0_ctx, sizeof(X0ChainCtx));
+    if(e==cudaSuccess) e = cudaMalloc(&h->x0_votes, 2*X0_CTRL_HISTORY);
     if(e==cudaSuccess) e = cudaFuncSetAttribute(pcm16x0_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227*1024);
     if(e==cudaSuccess) e = cudaMalloc(&h->p1_stats_dev, 4*sizeof(unsigned long long));
     if(e==cudaSuccess) e = cudaMallocHost(&h->p1_stats_host, 4*sizeof(unsigned long long));
@@ -1019,7 +1022,7 @@ void sdv_destroy(sdv_handle *h)
     cudaFree(h->cwd_spec_dev); cudaFree(h->cwd_status); cudaFree(h->cwd_scan_dev); cudaFree(h->cwd_plan_dev); cudaFree(h->blk_scratch); cudaFree(h->fres_dev);
     cudaFree(h->luma_dev); cudaFree(h->recs_dev); cudaFree(h->smp_dev); cudaFree(h->sfl_dev);
     cudaFreeHost(h->hdr_host); cudaFreeHost(h->fu_host); cudaFree(h->spec_fu);
-    cudaFree(h->p1_scan); cudaFree(h->p1_presets); cudaFree(h->p1_clean); cudaFree(h->p1_bw); cudaFree(h->p1_ctx); cudaFree(h->x0_ctx);
+    cudaFree(h->p1_scan); cudaFree(h->p1_presets); cudaFree(h->p1_clean); cudaFree(h->p1_bw); cudaFree(h->p1_ctx); cudaFree(h->x0_ctx); cudaFree(h->x0_votes);
     cudaFree(h->p1_stats_dev); cudaFreeHost(h->p1_stats_host); cudaFree(h->p1_sub);
     for(int i=0;i<2;i++) if(h->ev_sync[i]) cudaEventDestroy(h->ev_sync[i]);
     if(h->ev_lazy) cudaEventDestroy(h->ev_lazy);
@@ -1064,6 +1067,15 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
 {
     const bool x0 = (cfg->pcm_type==SDV_TYPE_PCM16X0);      // PCM-16x0: three sub-line records per video line
     if(W<(x0 ? (int)X0L_BITS : (int)P1_BITS)) return fail(h, SDV_ERR_ARG, "line shorter than the PCM bit cells", cudaSuccess);
+    // reserved[3] bit 0: this call continues the file of the previous PCM call on the handle: the chain state in p1_ctx / x0_ctx
+    // (Binarizer presets, coordinate histories, prescan_ref, the running pair G) goes on, and frame 0 is not the file's first
+    const int key_mode = cfg->mode|((cfg->check_line_dup ? 1 : 0)<<8);
+    const bool cont = (cfg->reserved[3]&1)!=0;
+    if(cont&&!(h->pcm_open&&(h->pcm_type==cfg->pcm_type)&&(h->pcm_H==H)&&(h->pcm_W==W)&&(h->pcm_mode==key_mode)))
+        return fail(h, SDV_ERR_ARG, "sdv_bin_decode_frames: nothing to continue (no earlier call with this PCM type, geometry and mode on the handle)", cudaSuccess);
+    if(cont&&(((int)cfg->reserved[0]|((int)cfg->reserved[1]<<8))>1))
+        return fail(h, SDV_ERR_ARG, "sdv_bin_decode_frames: a continuing PCM-1 / PCM-16x0 call decodes one file (chain_segments must be 0 or 1)", cudaSuccess);
+    h->pcm_open = 0;
     int rc;
     if((rc = ensure(h, (void **)&h->p1_scan, &h->p1_scan_cap, (size_t)n_frames*P1_COORD_CHECK_LINES*sizeof(P1Preset)))) return rc;
     if((rc = ensure(h, (void **)&h->p1_presets, &h->p1_presets_cap, (size_t)n_frames*sizeof(P1Preset)))) return rc;
@@ -1072,11 +1084,11 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     const bool prescan = (cfg->mode!=SDV_MODE_DRAFT);
     if(prescan)
     {
-        if(x0) pcm16x0_prescan_kernel<<<n_frames*P1_COORD_CHECK_LINES, P1S_THREADS, 0, st>>>(luma_dev, H, W, (size_t)stride, n_frames, cfg->mode, h->p1_scan);
-        else pcm1_prescan_kernel<<<n_frames*P1_COORD_CHECK_LINES, P1S_THREADS, 0, st>>>(luma_dev, H, W, (size_t)stride, n_frames, cfg->mode, h->p1_scan);
+        if(x0) pcm16x0_prescan_kernel<<<n_frames*P1_COORD_CHECK_LINES, P1S_THREADS, 0, st>>>(luma_dev, H, W, (size_t)stride, n_frames, cfg->mode, !cont, h->p1_scan);
+        else pcm1_prescan_kernel<<<n_frames*P1_COORD_CHECK_LINES, P1S_THREADS, 0, st>>>(luma_dev, H, W, (size_t)stride, n_frames, cfg->mode, !cont, h->p1_scan);
         h->stats.kernel_launches++;
     }
-    pcm1_preset_kernel<<<(n_frames+255)/256, 256, 0, st>>>(h->p1_scan, n_frames, H, cfg->mode, h->p1_presets);
+    pcm1_preset_kernel<<<(n_frames+255)/256, 256, 0, st>>>(h->p1_scan, n_frames, H, cfg->mode, !cont, h->p1_presets);
     h->stats.kernel_launches++;
     // bulk pass (only meaningful with per-frame presets, i.e. when the prescan runs)
     const BulkPlan bulk = bulk_plan(W, stride, luma_dev, P1_BULK_HEADER);
@@ -1088,7 +1100,7 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     {
         P1BulkParams bp;
         bp.luma = luma_dev; bp.H = H; bp.W = W; bp.stride = (size_t)stride; bp.n_frames = n_frames;
-        bp.presets = h->p1_presets; bp.line_dup = cfg->check_line_dup ? 1 : 0; bp.mode = cfg->mode;
+        bp.presets = h->p1_presets; bp.run_g = (x0&&cont) ? &h->x0_ctx->run_g : h->p1_presets; bp.line_dup = cfg->check_line_dup ? 1 : 0; bp.mode = cfg->mode;
         bp.recs = recs_dev; bp.aux = aux_dev; bp.clean = h->p1_clean; bp.frame_bw = h->p1_bw;
         bp.use_tma = bulk.use_tma; bp.warps = bulk.warps; bp.slot_bytes = bulk.slot_bytes;
         int grid = (n_frames+bulk.warps-1)/bulk.warps;
@@ -1105,7 +1117,7 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     {
         X0ChainParams xp;
         xp.luma = luma_dev; xp.H = H; xp.W = W; xp.stride = (size_t)stride; xp.n_frames = n_frames;
-        xp.mode = cfg->mode; xp.line_dup = cfg->check_line_dup ? 1 : 0; xp.use_bulk = use_bulk ? 1 : 0;
+        xp.mode = cfg->mode; xp.line_dup = cfg->check_line_dup ? 1 : 0; xp.use_bulk = use_bulk ? 1 : 0; xp.cont = cont ? 1 : 0;
         xp.scan = h->p1_scan; xp.presets = h->p1_presets; xp.clean = h->p1_clean; xp.frame_bw = h->p1_bw;
         xp.recs = recs_dev; xp.aux = aux_dev; xp.ctx = h->x0_ctx; xp.stats = h->p1_stats_dev;
         pcm16x0_chain_kernel<<<1, P1L_THREADS, sizeof(X0ChainCtx), st>>>(xp);
@@ -1114,7 +1126,7 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     {
     P1ChainParams cp;
     cp.luma = luma_dev; cp.H = H; cp.W = W; cp.stride = (size_t)stride; cp.n_frames = n_frames;
-    cp.mode = cfg->mode; cp.line_dup = cfg->check_line_dup ? 1 : 0; cp.use_bulk = use_bulk ? 1 : 0;
+    cp.mode = cfg->mode; cp.line_dup = cfg->check_line_dup ? 1 : 0; cp.use_bulk = use_bulk ? 1 : 0; cp.cont = cont ? 1 : 0;
     cp.presets = h->p1_presets; cp.clean = h->p1_clean; cp.frame_bw = h->p1_bw;
     cp.recs = recs_dev; cp.aux = aux_dev; cp.ctx = h->p1_ctx; cp.stats = h->p1_stats_dev;
     pcm1_chain_kernel<<<1, P1L_THREADS, sizeof(P1ChainCtx), st>>>(cp);
@@ -1129,6 +1141,7 @@ static int p1_decode_frames(sdv_handle *h, const sdv_bin_config *cfg, const uint
     h->stats.lines_fast = h->p1_stats_host[2]*(uint64_t)H*(x0 ? 3 : 1);
     if(x0) h->stats.lines_total = (uint64_t)n_frames*H*3;
     h->acc_launches += h->stats.kernel_launches;
+    h->pcm_open = 1; h->pcm_type = cfg->pcm_type; h->pcm_H = H; h->pcm_W = W; h->pcm_mode = key_mode;
     return SDV_OK;
 }
 
@@ -1201,7 +1214,7 @@ int sdv_bin_set_fine_settings(sdv_handle *h, const sdv_bin_preset *in)
     f.min_ref_lvl = in->min_ref_lvl; f.max_ref_lvl = in->max_ref_lvl; f.min_valid_crcs = in->min_valid_crcs;
     f.mark_max_dist = in->mark_max_dist; f.left_bit_pick = in->left_bit_pick; f.right_bit_pick = in->right_bit_pick;
     f.en_coord_search = in->en_coord_search ? 1 : 0; f.en_first_line_dup = in->en_first_line_dup ? 1 : 0;
-    if(!fine_equal(f, h->fine)) { h->fine = f; h->warm_valid = 0; h->chain_open = 0; }     // presets found with other settings are no guess for these
+    if(!fine_equal(f, h->fine)) { h->fine = f; h->warm_valid = 0; h->chain_open = 0; h->pcm_open = 0; }     // presets found with other settings are no guess for these
     return SDV_OK;
 }
 
@@ -1835,6 +1848,19 @@ int sdv_pcm16x0_frames_to_samples(sdv_handle *h, const sdv_pcm16x0_config *cfg, 
     return sdv_pcm16x0_frames_to_samples_info(h, cfg, geo, recs_dev, n_frames, H, mask_seams_dev, samples_dev, sample_flags_dev, NULL, cuda_stream);
 }
 
+// The control-bit history of the PCM-16x0 stitch calls: every call leaves the votes of its file's last X0_CTRL_HISTORY frames in
+// one of the handle's two vote buffers; a call with continue_file votes with what the call before left, otherwise with none.
+static int x0_votes_begin(sdv_handle *h, const sdv_pcm16x0_config *cfg, int ei, const u8 **hist_in, u8 **hist_out)
+{
+    if(cfg->continue_file&&(h->x0_votes_open!=1+ei))
+        return fail(h, SDV_ERR_ARG, "PCM-16x0 stitcher: nothing to continue (continue_file without an earlier stitch call in this format on the handle)", cudaSuccess);
+    *hist_in = cfg->continue_file ? h->x0_votes+h->x0_votes_cur*X0_CTRL_HISTORY : NULL;
+    *hist_out = h->x0_votes+(1-h->x0_votes_cur)*X0_CTRL_HISTORY;
+    h->x0_votes_open = 0;
+    return SDV_OK;
+}
+static void x0_votes_end(sdv_handle *h, int ei) { h->x0_votes_cur = 1-h->x0_votes_cur; h->x0_votes_open = 1+ei; }
+
 int sdv_pcm16x0_frames_to_samples_info(sdv_handle *h, const sdv_pcm16x0_config *cfg, const sdv_pcm16x0_geometry *geo, const sdv_line_rec *recs_dev,
                                        int n_frames, int H, const uint8_t *mask_seams_dev, int16_t *samples_dev, uint8_t *sample_flags_dev,
                                        sdv_pcm16x0_frame_info *info_dev, void *cuda_stream)
@@ -1845,23 +1871,27 @@ int sdv_pcm16x0_frames_to_samples_info(sdv_handle *h, const sdv_pcm16x0_config *
     if(n_frames==0) return SDV_OK;
     if(!recs_dev||!samples_dev||((uintptr_t)recs_dev%16)||((uintptr_t)samples_dev%2))
         return fail(h, SDV_ERR_ARG, "sdv_pcm16x0_frames_to_samples: null or misaligned buffer", cudaSuccess);
+    const int ei = cfg->ei_format ? 1 : 0;
+    const u8 *hist_in = NULL; u8 *hist_out = NULL;
+    { const int rc = x0_votes_begin(h, cfg, ei, &hist_in, &hist_out); if(rc) return rc; }
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
     X0Cfg c; c.ignore_crc = cfg->ignore_crc; c.force_check = cfg->force_check; c.p_corr = cfg->p_corr;
     timing_flush(h, 1);
     cudaEventRecord(h->ev[2], st);
     pcm16x0_stitch_kernel<<<n_frames, 512, 0, st>>>(recs_dev, n_frames, H, geo->bff, geo->top_padding_odd, geo->top_padding_even, c,
-                                                    geo->broken_mask_dur, mask_seams_dev, samples_dev, sample_flags_dev, info_dev, cfg->ei_format ? 1 : 0);
+                                                    geo->broken_mask_dur, mask_seams_dev, samples_dev, sample_flags_dev, info_dev, ei, hist_in, hist_out);
     cudaEventRecord(h->ev[3], st);
     h->ev_set[1] = 1; h->ev_units[1] = (uint64_t)n_frames*X0S_BLOCKS_FRAME;
     h->acc_launches += 1;
     if(info_dev)
     {
         if((uintptr_t)info_dev%2) return fail(h, SDV_ERR_ARG, "sdv_pcm16x0_frames_to_samples_info: misaligned info", cudaSuccess);
-        pcm16x0_ctrl_history_kernel<<<(unsigned)((n_frames+255)/256), 256, 0, st>>>(info_dev, n_frames);
+        pcm16x0_ctrl_history_kernel<<<(unsigned)((n_frames+255)/256), 256, 0, st>>>(info_dev, n_frames, hist_in);
         h->acc_launches += 1;
     }
     CK(cudaGetLastError());
+    x0_votes_end(h, ei);
     return SDV_OK;
 }
 
@@ -1874,14 +1904,18 @@ int sdv_pcm16x0_frames_to_samples_auto(sdv_handle *h, const sdv_pcm16x0_config *
     if(n_frames==0) return SDV_OK;
     if(!recs_dev||!samples_dev||((uintptr_t)recs_dev%16)||((uintptr_t)samples_dev%2)||((uintptr_t)info_dev%2))
         return fail(h, SDV_ERR_ARG, "sdv_pcm16x0_frames_to_samples_auto: null or misaligned buffer", cudaSuccess);
+    if(cfg->continue_file&&file_start)
+        return fail(h, SDV_ERR_ARG, "sdv_pcm16x0_frames_to_samples_auto: continue_file with file_start (a call either opens the file or continues it)", cudaSuccess);
+    const int ei = cfg->ei_format ? 1 : 0;
+    const u8 *hist_in = NULL; u8 *hist_out = NULL;
+    int rc;
+    if((rc = x0_votes_begin(h, cfg, ei, &hist_in, &hist_out))) return rc;
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    int rc;
     if((rc = ensure(h, (void **)&h->x0_scan, &h->x0_scan_cap, 2*(size_t)n_frames*sizeof(X0PadScan)))) return rc;
     if((rc = ensure(h, (void **)&h->x0_geo, &h->x0_geo_cap, 2*(size_t)n_frames*sizeof(X0FieldGeo)))) return rc;
     if((rc = ensure(h, (void **)&h->x0_mask, &h->x0_mask_cap, (size_t)n_frames+16))) return rc;
     X0Cfg c; c.ignore_crc = cfg->ignore_crc; c.force_check = cfg->force_check; c.p_corr = cfg->p_corr;
-    const int ei = cfg->ei_format ? 1 : 0;
     // a change of format drops the padding history (PCM16X0DataStitcher::setFormat -> resetState, 5456-5490, 5671-5676)
     if(file_start||(h->x0_pads_open!=1+ei)) h->x0_pads.reset();
     h->x0_pads.p_corr = cfg->p_corr!=0;
@@ -1925,17 +1959,18 @@ int sdv_pcm16x0_frames_to_samples_auto(sdv_handle *h, const sdv_pcm16x0_config *
     timing_flush(h, 1);
     cudaEventRecord(h->ev[2], st);
     pcm16x0_stitch_geo_kernel<<<n_frames, 512, 0, st>>>(recs_dev, n_frames, H, geo->bff, h->x0_geo, c, geo->broken_mask_dur, h->x0_mask,
-                                                        samples_dev, sample_flags_dev, info_dev, ei);
+                                                        samples_dev, sample_flags_dev, info_dev, ei, hist_in, hist_out);
     cudaEventRecord(h->ev[3], st);
     h->ev_set[1] = 1; h->ev_units[1] = (uint64_t)n_frames*X0S_BLOCKS_FRAME;
     h->acc_launches += 1;
     if(info_dev)
     {
-        pcm16x0_ctrl_history_kernel<<<(unsigned)((n_frames+255)/256), 256, 0, st>>>(info_dev, n_frames);
+        pcm16x0_ctrl_history_kernel<<<(unsigned)((n_frames+255)/256), 256, 0, st>>>(info_dev, n_frames, hist_in);
         h->acc_launches += 1;
     }
     CK(cudaStreamSynchronize(st));          // fg / mask are host vectors: the copies must be done before they go away
     CK(cudaGetLastError());
+    x0_votes_end(h, ei);
     return SDV_OK;
 }
 

@@ -93,7 +93,9 @@ class VideoToDigital:
                    on_first_frame=None, continue_file: bool = False, lazy: bool = False):
         """luma: CUDA uint8 [F, H, W] (interlaced frames).  Returns the record buffer uint8 [F*H, 32] (and the
         auxiliary buffer uint8 [F*H, 16]) in the reference's stream order: per frame, odd-field rows then even-field rows
-        (PCM-16x0: three sub-line records per row, [F*H*3, 32])."""
+        (PCM-16x0: three sub-line records per row, [F*H*3, 32]).  continue_file: the batch continues the file of the previous
+        call on the handle (same PCM type, geometry, mode and duplicate check), so a tape fed in batches decodes as in one call;
+        any format (STC-007, M2, PCM-1, PCM-16x0)."""
         luma = _dev_u8(luma)
         f, h, w = luma.shape
         n = f * h * (3 if self.pcm_type == capi.TYPE_PCM16X0 else 1)
@@ -103,7 +105,7 @@ class VideoToDigital:
         cfg = BinConfig(pcm_type=self.pcm_type, mode=self.mode, check_line_dup=int(self.check_line_dup))
         cfg.reserved[0], cfg.reserved[1] = self.chain_segments & 0xFF, (self.chain_segments >> 8) & 0xFF
         cfg.reserved[2] = (0 if self.warm_start else 1) | (0 if self.relay else 4) | (2 if lazy else 0)     # lazy: call verify() afterwards
-        cfg.reserved[3] = 1 if continue_file else 0          # the batch continues the file of the previous call (STC-007)
+        cfg.reserved[3] = 1 if continue_file else 0          # the batch continues the file of the previous call
         hook = None
         if on_first_frame is not None:
             # called as soon as the first frame's records are final (sdv_bin_on_first_frame): a shard starts its halo send here
@@ -351,16 +353,17 @@ class PCM16X0DataStitcher:
         self.broken_mask_dur = int(n)
 
     def doFrameReassemble(self, recs: torch.Tensor, n_frames: int, height: int, stream=None, mask_seams: torch.Tensor | None = None,
-                          want_info: bool = False):
+                          want_info: bool = False, continue_file: bool = False):
         """recs: the PCM-16x0 sub-line records of VideoToDigital.doBinarize; mask_seams: optional CUDA uint8 [n_frames], non-zero
         where the padding search was unsure about the frame.  Returns (samples int16 [n_frames*490, 6],
         flags uint8 [n_frames*490, 6]); with want_info also the control-bit decisions per frame (capi.PCM16X0_FRAME_INFO:
-        sample rate, emphasis, code as the reference writes them into the frame's sample pairs)."""
+        sample rate, emphasis, code as the reference writes them into the frame's sample pairs).  continue_file: the frames
+        continue those of the previous stitch call on the handle, whose control-bit votes then count for these."""
         recs = _dev_u8(recs)
         samples = torch.empty((n_frames * 490, 6), dtype=torch.int16, device=recs.device)
         flags = torch.empty((n_frames * 490, 6), dtype=torch.uint8, device=recs.device)
         cfg = capi.Pcm16x0Config(ignore_crc=int(self.ignore_crc), force_check=int(not self.ignore_crc), p_corr=int(self.p_corr),
-                                 ei_format=int(self.ei_format))
+                                 ei_format=int(self.ei_format), continue_file=int(continue_file))
         geo = capi.Pcm16x0Geometry(bff=int(self.field_order == self.ORDER_BFF), top_padding_odd=self.top_padding[0],
                                    top_padding_even=self.top_padding[1], broken_mask_dur=self.broken_mask_dur)
         info = torch.zeros((n_frames, capi.PCM16X0_FRAME_INFO.itemsize), dtype=torch.uint8, device=recs.device) if want_info else None
@@ -375,9 +378,11 @@ class PCM16X0DataStitcher:
 
 
 def pcm16x0_reassemble_auto(stitcher, recs: torch.Tensor, n_frames: int, height: int, stream=None, want_info: bool = False,
-                            file_start: bool = True, mask_seams: bool = True):
+                            file_start: bool = True, mask_seams: bool = True, continue_file: bool = False):
     """PCM16X0DataStitcher::doFrameReassemble with the vertical alignment searched as the reference does
     (sdv_pcm16x0_frames_to_samples_auto): findSIDataAlignment, or findEIFrameStitching after stitcher.setFormat(FORMAT_EI).
+    file_start=False keeps the padding history of the previous call; continue_file=True (with file_start=False) also its
+    control-bit history, so a tape stitched in batches gives the output of one call.
     Returns (samples int16 [n_frames*490, 6], flags uint8 [n_frames*490, 6], alignment capi.PCM16X0_ALIGNMENT [n_frames][, info])."""
     recs = _dev_u8(recs)
     dev = recs.device
@@ -386,7 +391,7 @@ def pcm16x0_reassemble_auto(stitcher, recs: torch.Tensor, n_frames: int, height:
     info = torch.empty((n_frames, capi.PCM16X0_FRAME_INFO.itemsize), dtype=torch.uint8, device=dev) if want_info else None
     align = np.zeros(max(n_frames, 1), capi.PCM16X0_ALIGNMENT)
     cfg = capi.Pcm16x0Config(ignore_crc=int(stitcher.ignore_crc), force_check=int(not stitcher.ignore_crc), p_corr=int(stitcher.p_corr),
-                             ei_format=int(getattr(stitcher, "ei_format", False)))
+                             ei_format=int(getattr(stitcher, "ei_format", False)), continue_file=int(continue_file))
     geo = capi.Pcm16x0Geometry(bff=int(stitcher.field_order == stitcher.ORDER_BFF), top_padding_odd=0, top_padding_even=0,
                                broken_mask_dur=int(stitcher.broken_mask_dur))
     rc = capi.lib().sdv_pcm16x0_frames_to_samples_auto(stitcher.handle.ptr, C.byref(cfg), C.byref(geo), C.c_void_p(recs.data_ptr()), n_frames, height,
@@ -578,15 +583,17 @@ def decode_tape_host(handle: capi.Handle, luma: np.ndarray, mode: int = MODE_NOR
 
 
 def decode_tape_host_pcm1(handle: capi.Handle, luma: np.ndarray, mode: int = MODE_NORMAL, check_line_dup: bool = True,
-                          bff: bool = False, ignore_crc: bool = False, offsets=None, want_recs: bool = False):
-    """sdv_pcm1_decode_tape_host: PCM-1 host luma [F, H, W] -> (samples int16 [F*2940], flags uint8 [F*2940], recs)."""
+                          bff: bool = False, ignore_crc: bool = False, offsets=None, want_recs: bool = False, continue_file: bool = False):
+    """sdv_pcm1_decode_tape_host: PCM-1 host luma [F, H, W] -> (samples int16 [F*2940], flags uint8 [F*2940], recs).
+    continue_file: the frames continue the file of the previous call on the handle (line decode and frame assembly)."""
     assert luma.dtype == np.uint8 and luma.ndim == 3 and luma.flags.c_contiguous
     f, h, w = luma.shape
     samples = np.empty(f * 2940, dtype=np.int16)
     flags = np.empty(f * 2940, dtype=np.uint8)
     recs = np.empty(f * h, dtype=LINE_REC) if want_recs else None
     bcfg = BinConfig(pcm_type=capi.TYPE_PCM1, mode=mode, check_line_dup=int(check_line_dup))
-    scfg = capi.Pcm1StitchConfig(ignore_crc=int(ignore_crc), bff=int(bff), file_start=1, manual_offset=int(offsets is not None),
+    bcfg.reserved[3] = int(continue_file)
+    scfg = capi.Pcm1StitchConfig(ignore_crc=int(ignore_crc), bff=int(bff), file_start=int(not continue_file), manual_offset=int(offsets is not None),
                                  odd_offset=(offsets or (0, 0))[0], even_offset=(offsets or (0, 0))[1])
     rc = capi.lib().sdv_pcm1_decode_tape_host(handle.ptr, C.byref(bcfg), C.byref(scfg), luma.ctypes.data_as(C.c_void_p), f, h, w,
                                               samples.ctypes.data_as(C.c_void_p), flags.ctypes.data_as(C.c_void_p),
@@ -597,15 +604,17 @@ def decode_tape_host_pcm1(handle: capi.Handle, luma: np.ndarray, mode: int = MOD
 
 def decode_tape_host_pcm16x0(handle: capi.Handle, luma: np.ndarray, mode: int = MODE_NORMAL, check_line_dup: bool = True,
                              bff: bool = False, ignore_crc: bool = False, p_corr: bool = True, top_padding=(5, 5),
-                             broken_mask_dur: int = 81, want_recs: bool = False):
-    """sdv_pcm16x0_decode_tape_host: PCM-16x0 (SI) host luma [F, H, W] -> (samples int16 [F*490, 6], flags uint8 [F*490, 6], recs)."""
+                             broken_mask_dur: int = 81, want_recs: bool = False, continue_file: bool = False):
+    """sdv_pcm16x0_decode_tape_host: PCM-16x0 (SI) host luma [F, H, W] -> (samples int16 [F*490, 6], flags uint8 [F*490, 6], recs).
+    continue_file: the frames continue the file of the previous call on the handle (line decode and control-bit history)."""
     assert luma.dtype == np.uint8 and luma.ndim == 3 and luma.flags.c_contiguous
     f, h, w = luma.shape
     samples = np.empty((f * 490, 6), dtype=np.int16)
     flags = np.empty((f * 490, 6), dtype=np.uint8)
     recs = np.empty(f * h * 3, dtype=LINE_REC) if want_recs else None
     bcfg = BinConfig(pcm_type=capi.TYPE_PCM16X0, mode=mode, check_line_dup=int(check_line_dup))
-    dcfg = capi.Pcm16x0Config(ignore_crc=int(ignore_crc), force_check=int(not ignore_crc), p_corr=int(p_corr))
+    bcfg.reserved[3] = int(continue_file)
+    dcfg = capi.Pcm16x0Config(ignore_crc=int(ignore_crc), force_check=int(not ignore_crc), p_corr=int(p_corr), continue_file=int(continue_file))
     geo = capi.Pcm16x0Geometry(bff=int(bff), top_padding_odd=top_padding[0], top_padding_even=top_padding[1], broken_mask_dur=broken_mask_dur)
     rc = capi.lib().sdv_pcm16x0_decode_tape_host(handle.ptr, C.byref(bcfg), C.byref(dcfg), C.byref(geo), luma.ctypes.data_as(C.c_void_p),
                                                  f, h, w, samples.ctypes.data_as(C.c_void_p), flags.ctypes.data_as(C.c_void_p),
