@@ -1368,9 +1368,10 @@ static int decode_frames_impl(sdv_handle *h, const sdv_bin_config *cfg, const ui
     // (consecutive pieces of a capture share levels and geometry).  The bulk kernel is launched with them on a second
     // stream, concurrently with the chain kernel that derives the true presets from the first frame; the guess is kept
     // only if the chain kernel arrives at exactly the same presets after exactly one frame, otherwise everything is
-    // redone without it.  Scheduling only: results never depend on the guess.
+    // redone without it.  Scheduling only: results never depend on the guess.  Not on a call that continues the file: its chain
+    // kernel advances the file's chain state in place, so a wrong guess could not start the call over from that state.
     bool warm_pending = false;
-    if(h->warm_valid&&(h->warm_H==H)&&(h->warm_W==W)&&(h->warm_mode==(cfg->mode|(dup_flags<<8)))&&(n_frames>1)&&!(cfg->reserved[2]&1))
+    if(h->warm_valid&&(h->warm_H==H)&&(h->warm_W==W)&&(h->warm_mode==(cfg->mode|(dup_flags<<8)))&&(n_frames>1)&&!(cfg->reserved[2]&1)&&!cont)
     {
         CK(cudaEventRecord(h->ev_sync[0], st));
         CK(cudaStreamWaitEvent(h->copy_stream, h->ev_sync[0], 0));
