@@ -320,6 +320,19 @@ SDV_API int sdv_stc007_stitch_frames(sdv_handle *h, const sdv_deint_config *cfg,
                                      sdv_block_rec *blocks_dev, int16_t *samples_dev, uint8_t *sample_flags_dev,
                                      int *n_blocks_out, int *n_frames_done, sdv_stc007_frame_info *info_host, void *cuda_stream);
 
+/* ---- the open file of sdv_stc007_stitch_frames as a portable blob of sdv_stc007_stitch_state_bytes() bytes in device memory
+ * (4-byte aligned): the previous frame's state, the field-order and resolution histories, the broken-block countdown, the 112
+ * queued lines with their CWD-patched copies, and whether CWD and resolution detection were on.  The form is canonical -- rings
+ * rotated to position 0, frame numbers counted from the first frame after the state, unused bytes zero -- so two states with the
+ * same future compare equal byte for byte.  _save: the handle's open file (a call with file_end = 0 left it; SDV_ERR_ARG without
+ * one) -> state_dev, one launch on the stream, no synchronisation.  _load: state_dev -> the handle's open file, so the next call
+ * may pass file_start = 0, on this handle or another one on any device; synchronises the stream.  A blob of another magic,
+ * version or size fails with SDV_ERR_ARG, and so does a continuing call after a load whose sdv_deint_config.cwd or detected
+ * resolution (resolution_16bit = 2) differs from the saved state's.  file_start = 1 still resets everything. */
+SDV_API int sdv_stc007_stitch_state_bytes(void);
+SDV_API int sdv_stc007_stitch_state_save(sdv_handle *h, void *state_dev, void *cuda_stream);
+SDV_API int sdv_stc007_stitch_state_load(sdv_handle *h, const void *state_dev, void *cuda_stream);
+
 /* ---- whole path with HOST buffers (what the reference-facing plugin calls): H2D luma, line decode, assembly,
  * deinterleave + P/Q, D2H samples.  samples_host [n_blocks][6] int16, flags_host [n_blocks][6] (may be NULL),
  * recs_host [n_frames*H] (may be NULL). */

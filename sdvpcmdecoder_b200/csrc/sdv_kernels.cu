@@ -863,6 +863,8 @@ struct sdv_handle
     sdv_stitch_stats *sstat_dev; size_t sstat_cap;
     sdv_line_rec *carry_dev[2]; i32 *carry_meta_dev[2]; int carry_cur, carry_valid;   // the 112 lines a call leaves in the queue for the next
     StitchCarry st_carry; int st_frame_base; int st_countdown; ResChain st_res;
+    int st_flags;               // SB_FLAG_* of the call that left the open file (what a saved state records)
+    int st_loaded;              // the open file came from sdv_stc007_stitch_state_load: the next call must match st_flags
     u8 *fres_dev; size_t fres_cap;  // detected resolution per field + the four modes per frame
     // CWD
     u8 *cwd_scan_dev; size_t cwd_scan_cap; u8 *cwd_plan_dev; size_t cwd_plan_cap; int *cwd_status;
@@ -2189,6 +2191,9 @@ int sdv_stc007_stitch_frames(sdv_handle *h, const sdv_deint_config *cfg, const s
     std::vector<u8> cwd_patch;
     if((n_frames>0)&&(!recs_dev||((uintptr_t)recs_dev%16))) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_frames: null or misaligned records", cudaSuccess);
     if((!scfg->file_start)&&(!h->carry_valid)) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_frames: nothing to continue (file_start = 0 on a handle without an open file)", cudaSuccess);
+    const int st_flags = (cwd ? SB_FLAG_CWD : 0)|(res_auto ? SB_FLAG_RES_AUTO : 0);
+    if((!scfg->file_start)&&h->st_loaded&&(h->st_flags!=st_flags))
+        return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_frames: the loaded state was saved with other CWD / resolution detection settings", cudaSuccess);
     CK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;
     if(n_blocks_out) *n_blocks_out = 0;
@@ -2447,12 +2452,14 @@ int sdv_stc007_stitch_frames(sdv_handle *h, const sdv_deint_config *cfg, const s
         h->cwd_carry_valid = (cwd&&cwd_last_dirty&&(n_blocks>0)) ? 1 : ((n_done>0) ? 0 : h->cwd_carry_valid);
         h->st_carry = sx.st; h->st_frame_base += n_done;
         h->st_countdown = ((n_blocks>0)&&(cfg->broken_mask_dur>0)) ? h->win_state_host[1] : h->st_countdown;
+        h->st_flags = st_flags;
     }
     else
     {
         CK(cudaStreamSynchronize(st));
         h->carry_valid = 0; h->st_countdown = 0; h->cwd_carry_valid = 0;
     }
+    h->st_loaded = 0;
     CK(cudaGetLastError());
     if(cwd)
     {
@@ -2462,6 +2469,90 @@ int sdv_stc007_stitch_frames(sdv_handle *h, const sdv_deint_config *cfg, const s
     }
     if(n_blocks_out) *n_blocks_out = (int)n_blocks;
     if(n_frames_done) *n_frames_done = n_done;
+    return SDV_OK;
+}
+
+// ---- the open file of the stitcher as a blob (layout: SB_* in stc007_stitch.cuh)
+static_assert((sizeof(CwdLine)==32)&&(offsetof(CwdLine, frame)==28)&&(sizeof(sdv_line_rec)==32), "blob layout of the carried lines");
+static void sb_put(StitchBlobHdr *o, int at, const void *p, size_t n) { memcpy((u8 *)o->w+at, p, n); }
+static const u8 *sb_at(const StitchBlobHdr &o, int at) { return (const u8 *)o.w+at; }
+
+static StitchBlobHdr stitch_state_encode(const sdv_handle *h)
+{
+    StitchBlobHdr o; memset(&o, 0, sizeof(o));
+    const u32 magic = SB_MAGIC, size = SB_BYTES; const u16 version = SB_VERSION, flags = (u16)h->st_flags;
+    const i32 n_carry = h->carry_valid, n_cwd = h->cwd_carry_valid ? h->carry_valid : 0, countdown = h->st_countdown;
+    sb_put(&o, SBH_MAGIC, &magic, 4); sb_put(&o, SBH_VERSION, &version, 2); sb_put(&o, SBH_FLAGS, &flags, 2); sb_put(&o, SBH_SIZE, &size, 4);
+    sb_put(&o, SBH_CARRY, &n_carry, 4); sb_put(&o, SBH_CWD_VALID, &n_cwd, 4); sb_put(&o, SBH_COUNTDOWN, &countdown, 4);
+    const FrameSt &f = h->st_carry.f0;
+    const u16 w16[4] = { f.odd_lines, f.even_lines, f.inner_pad, f.outer_pad };
+    const u8 w8[13] = { f.order, (u8)f.order_preset, (u8)f.order_guessed, f.video_std, (u8)f.std_preset, (u8)f.inner_ok, (u8)f.outer_ok,
+                        (u8)f.inner_silence, (u8)f.outer_silence, f.tff_cnt, f.bff_cnt, f.odd_res, f.even_res };
+    sb_put(&o, SBH_F0, w16, 8); sb_put(&o, SBH_F0+8, w8, 13);
+    sb_put(&o, SBH_LAST_PAD, &h->st_carry.last_pad_counter, 1);
+    u8 *order = (u8 *)o.w+SBH_ORDER, *res = (u8 *)o.w+SBH_RES;     // the rings from their oldest entry on, position 0
+    for(int i=0;i<65;i++) { order[i] = h->st_carry.order_hist[(h->st_carry.order_pos+i)%65]; res[i] = h->st_res.hist[(h->st_res.pos+i)%65]; }
+    return o;
+}
+
+// Header -> handle state; false for a blob this build did not write (nothing is changed then).
+static bool stitch_state_decode(const StitchBlobHdr &o, sdv_handle *h)
+{
+    u32 magic, size; u16 version, flags; i32 n_carry, n_cwd, countdown;
+    memcpy(&magic, sb_at(o, SBH_MAGIC), 4); memcpy(&version, sb_at(o, SBH_VERSION), 2); memcpy(&flags, sb_at(o, SBH_FLAGS), 2);
+    memcpy(&size, sb_at(o, SBH_SIZE), 4); memcpy(&n_carry, sb_at(o, SBH_CARRY), 4); memcpy(&n_cwd, sb_at(o, SBH_CWD_VALID), 4);
+    memcpy(&countdown, sb_at(o, SBH_COUNTDOWN), 4);
+    if((magic!=SB_MAGIC)||(version!=SB_VERSION)||(size!=SB_BYTES)||(flags>3)) return false;
+    if((n_carry<1)||(n_carry>ST_TAIL)||((n_cwd!=0)&&(n_cwd!=n_carry))||((n_cwd!=0)&&!(flags&SB_FLAG_CWD))||(countdown<0)||(countdown>255)) return false;
+    u16 w16[4]; u8 w8[13];
+    memcpy(w16, sb_at(o, SBH_F0), 8); memcpy(w8, sb_at(o, SBH_F0+8), 13);
+    if((w8[0]>2)||(w8[3]>2)||(w8[11]>SDV_RES_MODE_16BIT)||(w8[12]>SDV_RES_MODE_16BIT)) return false;
+    for(int i : {1, 2, 4, 5, 6, 7, 8}) if(w8[i]>1) return false;
+    const u8 *order = sb_at(o, SBH_ORDER), *res = sb_at(o, SBH_RES);
+    for(int i=0;i<65;i++) if((order[i]>2)||(res[i]>2)) return false;
+    FrameSt &f = h->st_carry.f0;
+    f.odd_lines = w16[0]; f.even_lines = w16[1]; f.inner_pad = w16[2]; f.outer_pad = w16[3];
+    f.order = w8[0]; f.order_preset = w8[1]; f.order_guessed = w8[2]; f.video_std = w8[3]; f.std_preset = w8[4]; f.inner_ok = w8[5];
+    f.outer_ok = w8[6]; f.inner_silence = w8[7]; f.outer_silence = w8[8]; f.tff_cnt = w8[9]; f.bff_cnt = w8[10]; f.odd_res = w8[11]; f.even_res = w8[12];
+    h->st_carry.last_pad_counter = *sb_at(o, SBH_LAST_PAD);
+    memcpy(h->st_carry.order_hist, order, 65); h->st_carry.order_pos = 0;
+    memcpy(h->st_res.hist, res, 65); h->st_res.pos = 0;
+    h->st_countdown = countdown; h->carry_valid = n_carry; h->cwd_carry_valid = n_cwd ? 1 : 0;
+    h->st_frame_base = 0; h->st_flags = flags; h->st_loaded = 1;
+    return true;
+}
+
+int sdv_stc007_stitch_state_bytes(void) { return SB_BYTES; }
+
+int sdv_stc007_stitch_state_save(sdv_handle *h, void *state_dev, void *cuda_stream)
+{
+    if(!h) return SDV_ERR_ARG;
+    if(!state_dev||((uintptr_t)state_dev%4)) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_state_save: null or misaligned state buffer", cudaSuccess);
+    if(!h->carry_valid) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_state_save: no open file on the handle", cudaSuccess);
+    CK(cudaSetDevice(h->device));
+    const StitchBlobHdr hdr = stitch_state_encode(h);
+    const int c = h->carry_cur;
+    stitch_state_pack_kernel<<<(SB_BYTES/4+255)/256, 256, 0, (cudaStream_t)cuda_stream>>>(hdr, (const u32 *)h->carry_dev[c], h->carry_meta_dev[c],
+        (const u32 *)h->cwd_carry[c], h->carry_valid, h->cwd_carry_valid ? h->carry_valid : 0, h->st_frame_base+1, (u32 *)state_dev);
+    h->acc_launches += 1;
+    CK(cudaGetLastError());
+    return SDV_OK;
+}
+
+int sdv_stc007_stitch_state_load(sdv_handle *h, const void *state_dev, void *cuda_stream)
+{
+    if(!h) return SDV_ERR_ARG;
+    if(!state_dev||((uintptr_t)state_dev%4)) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_state_load: null or misaligned state buffer", cudaSuccess);
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    StitchBlobHdr hdr;
+    CK(cudaMemcpyAsync(&hdr, state_dev, sizeof(hdr), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if(!stitch_state_decode(hdr, h)) return fail(h, SDV_ERR_ARG, "sdv_stc007_stitch_state_load: not a stitcher state of this version", cudaSuccess);
+    const int c = h->carry_cur;
+    stitch_state_unpack_kernel<<<(SB_BYTES/4+255)/256, 256, 0, st>>>((const u32 *)state_dev, (u32 *)h->carry_dev[c], h->carry_meta_dev[c], (u32 *)h->cwd_carry[c], 1);
+    h->acc_launches += 1;
+    CK(cudaStreamSynchronize(st));
     return SDV_OK;
 }
 

@@ -416,4 +416,52 @@ SDV_HD bool stitch_block_in(const StitchMap &m, long long b, bool ignore_crc, Bl
     return masked;
 }
 
+// ------------------------------------------------------------------------------------------------ the carried state as a blob
+// sdv_stc007_stitch_state_save / _load: everything a call with file_start = 0 reads from the handle, in one canonical byte
+// layout, so that two states with the same future compare equal with memcmp.  The header (host part of the state: frame state,
+// histories rotated to position 0, countdown, counts) is built on the host; the line part moves on the device.  Frame numbers
+// are stored counted from the first frame after the state (that frame = 0); lines past the valid counts are zero.
+enum { SB_MAGIC = 0x53535453u /* "STSS" */, SB_VERSION = 1, SB_HDR = 256,
+       SB_RECS = SB_HDR,                        // ST_TAIL carried line records (sdv_line_rec, 32 bytes)
+       SB_META = SB_RECS+ST_TAIL*32,            // ST_TAIL (frame, line) pairs (i32)
+       SB_CWD = SB_META+ST_TAIL*8,              // ST_TAIL CWD-patched lines (CwdLine, 32 bytes, frame number in its last word)
+       SB_BYTES = SB_CWD+ST_TAIL*32 };
+// Header byte offsets.
+enum { SBH_MAGIC = 0, SBH_VERSION = 4, SBH_FLAGS = 6, SBH_SIZE = 8, SBH_CARRY = 12, SBH_CWD_VALID = 16, SBH_COUNTDOWN = 20,
+       SBH_F0 = 24 /* FrameSt: 4 x u16, then 13 x u8 */, SBH_LAST_PAD = 56, SBH_ORDER = 64 /* 65 entries */, SBH_RES = 132 /* 65 entries */ };
+enum { SB_FLAG_CWD = 1, SB_FLAG_RES_AUTO = 2 };
+struct StitchBlobHdr { u32 w[SB_HDR/4]; };
+
+#if defined(__CUDACC__)
+// Blob word k <- header | records | (frame - base, line) | CWD lines with frame - base.  n_carry / n_cwd: valid lines.
+__global__ void __launch_bounds__(256) stitch_state_pack_kernel(StitchBlobHdr hdr, const u32 *recs, const i32 *meta, const u32 *cwd,
+                                                                int n_carry, int n_cwd, i32 base, u32 *blob)
+{
+    for(int k=blockIdx.x*blockDim.x+threadIdx.x;k<SB_BYTES/4;k+=gridDim.x*blockDim.x)
+    {
+        u32 v = 0;
+        if(k<SB_RECS/4)
+        {   // (selected, not indexed: a dynamic index into a kernel parameter would put it on the stack)
+#pragma unroll
+            for(int j=0;j<SB_HDR/4;j++) if(j==k) v = hdr.w[j];
+        }
+        else if(k<SB_META/4) { const int i = k-SB_RECS/4; if(i/8<n_carry) v = recs[i]; }
+        else if(k<SB_CWD/4) { const int i = k-SB_META/4; if(i/2<n_carry) v = (i&1) ? (u32)meta[i] : (u32)(meta[i]-base); }
+        else { const int i = k-SB_CWD/4; if(i/8<n_cwd) v = ((i&7)==7) ? (u32)((i32)cwd[i]-base) : cwd[i]; }
+        blob[k] = v;
+    }
+}
+// The line part of a blob back into the handle's carry slot, frame numbers + base.
+__global__ void __launch_bounds__(256) stitch_state_unpack_kernel(const u32 *blob, u32 *recs, i32 *meta, u32 *cwd, i32 base)
+{
+    for(int k=SB_RECS/4+blockIdx.x*blockDim.x+threadIdx.x;k<SB_BYTES/4;k+=gridDim.x*blockDim.x)
+    {
+        const u32 v = blob[k];
+        if(k<SB_META/4) recs[k-SB_RECS/4] = v;
+        else if(k<SB_CWD/4) { const int i = k-SB_META/4; meta[i] = (i&1) ? (i32)v : (i32)v+base; }
+        else { const int i = k-SB_CWD/4; cwd[i] = ((i&7)==7) ? (u32)((i32)v+base) : v; }
+    }
+}
+#endif
+
 }   // namespace sdv

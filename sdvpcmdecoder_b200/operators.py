@@ -486,6 +486,24 @@ class STC007DataStitcher(_DeintSettings):
         self.handle.check(rc)
         return (blocks[:nb.value] if want_blocks else None), samples[:nb.value], flags[:nb.value], info[:nd.value]
 
+    def saveState(self, out: torch.Tensor | None = None, stream=None) -> torch.Tensor:
+        """The open file a doFrameReassembleAuto(file_end=False) call left on the handle, as a canonical uint8 CUDA tensor of
+        sdv_stc007_stitch_state_bytes() bytes (sdv_stc007_stitch_state_save): equal states give equal bytes.  No synchronisation."""
+        n = int(capi.lib().sdv_stc007_stitch_state_bytes())
+        if out is None:
+            out = torch.empty(n, dtype=torch.uint8, device=torch.device("cuda", self.handle.device))
+        out = _dev_u8(out)
+        assert out.numel() == n
+        self.handle.check(capi.lib().sdv_stc007_stitch_state_save(self.handle.ptr, C.c_void_p(out.data_ptr()), _stream_ptr(stream)))
+        return out
+
+    def loadState(self, state: torch.Tensor, stream=None):
+        """Make [state] (from saveState, on any handle) the open file of this handle: the next doFrameReassembleAuto(file_start=False)
+        continues it, with the CWD and resolution-detection settings it was saved with (sdv_stc007_stitch_state_load)."""
+        state = _dev_u8(state)
+        assert state.numel() == int(capi.lib().sdv_stc007_stitch_state_bytes())
+        self.handle.check(capi.lib().sdv_stc007_stitch_state_load(self.handle.ptr, C.c_void_p(state.data_ptr()), _stream_ptr(stream)))
+
     def geometry(self) -> Geometry:
         return Geometry(lines_per_field=LINES_PER_FIELD[self.video_std], lead_in=self.lead_in)
 

@@ -163,6 +163,173 @@ class CountdownHandoff:
         raise RuntimeError("countdown hand-off did not settle")
 
 
+# ---- the own-alignment stitcher (STC007DataStitcher.doFrameReassembleAuto) over frame shards
+#
+# Its carried state (previous frame, 65-entry order / resolution histories, countdown, the last 112 queued lines) depends on
+# the whole tape before a shard, so each shard guesses it and the guesses are verified: rank g stitches the K frames in front of
+# its first frame from a file start (a warm-up whose output is thrown away), continues over its own frames from the state that
+# leaves, then compares that state with the end state of rank g-1.  The states are canonical blobs (saveState), so equality is
+# byte equality.  A rank whose guess was wrong loads the true state and runs again; rank 0 is exact, so after round r the
+# first r+1 shards are final: at most [world] rounds.
+
+STITCH_WARMUP_FRAMES = 70       # the 65-entry histories refill, plus a margin
+
+
+class DistTransport:
+    """Records and state blobs between the ranks of a torch.distributed process group (NCCL from device memory, gloo on CPUs)."""
+
+    def __init__(self, rank: int | None = None, world: int | None = None):
+        self.rank = dist.get_rank() if rank is None else rank
+        self.world = dist.get_world_size() if world is None else world
+
+    def send(self, t: torch.Tensor, dst: int):
+        dist.send(t.contiguous(), dst)
+
+    def recv(self, t: torch.Tensor, src: int):
+        dist.recv(t, src)
+
+    def all_gather(self, t: torch.Tensor) -> torch.Tensor:
+        out = [torch.empty_like(t) for _ in range(self.world)]
+        dist.all_gather(out, t.contiguous())
+        return torch.stack(out)
+
+
+class LocalTransport:
+    """Ranks as threads of one process (several handles on one GPU): what DistTransport does, through in-process mailboxes.
+    LocalTransport(world).run(fn) calls fn(transport of rank r) for every rank at once and returns the results in rank order."""
+
+    def __init__(self, world: int, timeout: float = 600.0):
+        import queue
+        import threading
+        self.world, self.timeout = world, timeout
+        self._boxes = {(s, d): queue.Queue() for s in range(world) for d in range(world)}
+        self._barrier = threading.Barrier(world, timeout=timeout)
+        self._slots = [None] * world
+
+    class _Rank:
+        def __init__(self, hub, rank):
+            self.hub, self.rank, self.world = hub, rank, hub.world
+
+        def send(self, t, dst):
+            self.hub._boxes[(self.rank, dst)].put(t.clone())
+
+        def recv(self, t, src):
+            import queue
+            import time
+            end = time.monotonic() + self.hub.timeout
+            while True:     # (in slices, so that a rank that failed ends the others' waits)
+                if self.hub._barrier.broken:
+                    raise RuntimeError("another rank failed")
+                try:
+                    t.copy_(self.hub._boxes[(src, self.rank)].get(timeout=0.5))
+                    return
+                except queue.Empty:
+                    if time.monotonic() > end:
+                        raise
+
+        def all_gather(self, t):
+            self.hub._slots[self.rank] = t.clone()
+            self.hub._barrier.wait()
+            out = torch.stack(self.hub._slots)
+            self.hub._barrier.wait()
+            return out
+
+    def run(self, fn):
+        import threading
+        results, errors = [None] * self.world, []
+
+        def body(r):
+            try:
+                results[r] = fn(LocalTransport._Rank(self, r))
+            except BaseException as e:      # noqa: BLE001 -- re-raised below; the others must not wait for this rank
+                errors.append(e)
+                self._barrier.abort()
+        threads = [threading.Thread(target=body, args=(r,)) for r in range(self.world)]
+        for t in threads:
+            t.start()
+        for t in threads:
+            t.join()
+        if errors:
+            raise errors[0]
+        return results
+
+
+def stitch_shard(stitcher, recs: torch.Tensor, n_frames: int, lines_per_frame: int, transport,
+                 warmup: int = STITCH_WARMUP_FRAMES, edges=None, **stitch_kw):
+    """Own-alignment stitching of this rank's frames [a, b) = frame_range(n_frames, rank, world) so that the shards' outputs
+    concatenate to one doFrameReassembleAuto call over the whole tape.
+
+    stitcher: an STC007DataStitcher on this rank's handle (doFrameReassembleAuto, saveState, loadState); recs: the line records of
+    frames [a, b) ([(b-a)*lines_per_frame, 32]); transport: DistTransport or LocalTransport rank; edges: world+1 frame indices
+    [0, a_1, .., n_frames] for shards other than frame_range's; stitch_kw goes to doFrameReassembleAuto.
+    Steps: (1) receive the records of the [warmup] frames before a from rank-1 (passed along when shards are shorter) and of
+    frame b from rank+1, the frame the stitcher looks ahead to; (2) warm-up: frames [a-warmup, a] from a file start,
+    output discarded, its end state is the guess at a (exact when a-warmup <= 0); (3) continue over [a, b] (the last rank over [a, n)
+    with file_end), save the end state; (4) all-gather (state started from, end state) of every rank, redo the ranks whose start
+    differs from their predecessor's end, repeat until none does.
+    Returns (the doFrameReassembleAuto output of the final run, stats): the shard's blocks start at the first of the 112 lines
+    carried in from rank-1 (rank 0: at the lead-in); stats = warmup_frames, warmup_s, total_s, rounds (the ranks redone in each
+    round), redone (runs of this rank after the first)."""
+    import time
+    rank, world, H = transport.rank, transport.world, lines_per_frame
+    if edges is None:
+        edges = [frame_range(n_frames, g, world)[0] for g in range(world)] + [n_frames]
+    if len(edges) != world + 1 or edges[0] != 0 or edges[-1] != n_frames or any(edges[g + 1] <= edges[g] for g in range(world)):
+        raise ValueError("every shard needs at least one frame, and the shards must cover the tape")
+    a, b = edges[rank], edges[rank + 1]
+    if recs.shape[0] != (b - a) * H:
+        raise ValueError("recs must hold the line records of this rank's frames")
+    t0 = time.perf_counter()
+    # (1) records
+    k = min(warmup, a)
+    head = recs.new_empty((k * H,) + tuple(recs.shape[1:]))
+    if rank > 0:
+        transport.recv(head, rank - 1)
+    if rank < world - 1:
+        k_next = min(warmup, b)
+        transport.send(torch.cat([head, recs])[(k + b - a - k_next) * H:], rank + 1)
+    if rank > 0:
+        transport.send(recs[:H], rank - 1)
+    last = rank == world - 1
+    run_recs = recs
+    if not last:
+        ahead = recs.new_empty((H,) + tuple(recs.shape[1:]))
+        transport.recv(ahead, rank + 1)
+        run_recs = torch.cat([recs, ahead])
+    # (2) warm-up
+    if rank > 0:
+        stitcher.doFrameReassembleAuto(torch.cat([head, recs[:H]]), k + 1, H, file_start=True, file_end=False, **stitch_kw)
+        start = stitcher.saveState()
+    t_warm = time.perf_counter() - t0
+
+    # (3) the shard
+    def run():
+        out = stitcher.doFrameReassembleAuto(run_recs, run_recs.shape[0] // H, H, file_start=(rank == 0), file_end=last, **stitch_kw)
+        return out, (None if last else stitcher.saveState())
+    out, end = run()
+    rounds, redone = [], 0
+    if world == 1:
+        return out, {"warmup_frames": 0, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone}
+    # (4) verify / redo (nobody compares with rank 0's start or the last rank's end: placeholders of the blob's shape)
+    if rank == 0:
+        start = end
+    if last:
+        end = start
+    for _ in range(world + 1):
+        both = transport.all_gather(torch.stack([start, end]))
+        bad = [g for g in range(1, world) if not torch.equal(both[g, 0], both[g - 1, 1])]
+        if not bad:
+            return out, {"warmup_frames": k, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone}
+        rounds.append(bad)
+        if rank in bad:
+            start = both[rank - 1, 1].clone()
+            stitcher.loadState(start)
+            out, end = run()
+            end = start if last else end
+            redone += 1
+    raise RuntimeError("stitcher state hand-off did not settle")
+
+
 def bind_to_gpu_numa_node(device_index: int):
     """Pin this process to the CPUs of the NUMA node the GPU hangs off, so that host buffers allocated afterwards (the
     pinned luma / sample buffers of the host entry points) are local to the GPU's PCIe root: with one process per GPU
