@@ -210,6 +210,28 @@ SDV_API int sdv_bin_set_fine_settings(sdv_handle *h, const sdv_bin_preset *in);
  * still be the caller's) and everything computed from the records since has to be computed again.  No-op without a pending call. */
 SDV_API int sdv_bin_decode_verify(sdv_handle *h, int *redone);
 
+/* ---- the open file of the line decode as a portable blob of sdv_bin_chain_state_bytes() bytes in device memory (4-byte aligned),
+ * so that a decode can be checkpointed and resumed on another handle or device, or split over frame shards with a verified
+ * hand-off (sharding.decode_shard).  The blob is canonical: equal bytes mean that every later call decodes the same records and
+ * aux.  Layout (little endian; chain_state.cuh CS_* / CSH_* / CSB_*):
+ *   [0, 64)    header: magic "SDCS" (u32), version (u16), PCM type (u16), size (u32), H, W (u16), mode, duplicate-line check,
+ *              M2 sample format (u8), then at 32 the handle's sdv_bin_preset fine settings, verbatim;
+ *   [64, 292)  the chain state at the frame boundary: the Binarizer presets (BinState), field state, duplicate check, M2 flag,
+ *              the prescan's reference level (PCM-1 / PCM-16x0), the history counts, the words of the previous line, the frame
+ *              average and the 9-line (PCM-16x0: 27 sub-line) and 16-frame coordinate histories;
+ *   the rest zero, as are history entries past their counts.  Counters and PCM-16x0's running pair G of the bulk pass
+ *   (scheduling only, derived from the history on load) are not part of it.
+ * _save: the open file of [pcm_type]'s kind (STC-007 / M2: the one sdv_bin_decode_frames keeps for those two, PCM-1 / PCM-16x0:
+ * the other) -> state_dev, one launch on the stream, no synchronisation.  _load: checks the blob on the host, then makes it the
+ * open file of its kind on this handle, keyed by the blob's PCM type, H, W, mode and duplicate check: the next call with
+ * sdv_bin_config.reserved[3] bit 0 and that key continues it exactly as the saved handle would have; synchronises the stream.
+ * SDV_ERR_ARG: save without an open file of that kind; save or load while a lazy call awaits sdv_bin_decode_verify; load of a blob
+ * with a wrong magic, version or size, an out-of-range field or bytes not in canonical form; load when the handle's fine
+ * settings differ from the blob's. */
+SDV_API int sdv_bin_chain_state_bytes(void);
+SDV_API int sdv_bin_chain_state_save(sdv_handle *h, int pcm_type, void *state_dev, void *cuda_stream);
+SDV_API int sdv_bin_chain_state_load(sdv_handle *h, const void *state_dev, void *cuda_stream);
+
 /* ---- optional hook: [fn] is called from inside sdv_bin_decode_frames() (same thread) as soon as the records of the FIRST
  * frame are final -- on an STC-007 call with a warm handle that is while the bulk pass over the other frames is still
  * running on the device; on every other path it is called once before the function returns.  A frame-sharded decoder

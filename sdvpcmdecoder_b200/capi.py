@@ -128,7 +128,8 @@ EXPORTS = ("sdv_create", "sdv_destroy", "sdv_last_error", "sdv_version", "sdv_bi
            "sdv_pcm1_frames_to_samples", "sdv_pcm16x0_frames_to_samples", "sdv_pcm16x0_frames_to_samples_info", "sdv_pcm1_decode_tape_host", "sdv_pcm16x0_decode_tape_host",
            "sdv_stc007_stitch_frames", "sdv_stc007_stitch_block_bound", "sdv_stc007_countdown", "sdv_stc007_countdown_copy", "sdv_pcm16x0_frames_to_samples_auto",
            "sdv_bin_default_fine_settings", "sdv_bin_get_fine_settings", "sdv_bin_set_fine_settings", "sdv_bin_decode_verify", "sdv_stc007_fuse_next_decode",
-           "sdv_stc007_stitch_state_bytes", "sdv_stc007_stitch_state_save", "sdv_stc007_stitch_state_load")
+           "sdv_stc007_stitch_state_bytes", "sdv_stc007_stitch_state_save", "sdv_stc007_stitch_state_load",
+           "sdv_bin_chain_state_bytes", "sdv_bin_chain_state_save", "sdv_bin_chain_state_load")
 
 FIRST_FRAME_FN = C.CFUNCTYPE(None, C.c_void_p)
 _lib = None
@@ -187,6 +188,9 @@ def lib():
         l.sdv_stc007_stitch_state_bytes.argtypes = []
         l.sdv_stc007_stitch_state_save.argtypes = [vp, vp, vp]
         l.sdv_stc007_stitch_state_load.argtypes = [vp, vp, vp]
+        l.sdv_bin_chain_state_bytes.argtypes = []
+        l.sdv_bin_chain_state_save.argtypes = [vp, ci, vp, vp]
+        l.sdv_bin_chain_state_load.argtypes = [vp, vp, vp]
         _lib = l
     return _lib
 

@@ -21,6 +21,7 @@
 #include <new>
 #include <vector>
 #include <algorithm>
+#include <memory>
 #include "stc007_chain.cuh"
 #include "stc007_deint.cuh"
 #include "stc007_stitch_host.h"
@@ -35,6 +36,7 @@
 #include "pcm16x0_kernels.cuh"
 #include "pcm16x0_stitch.cuh"
 #include "pcm16x0_stitch_host.h"
+#include "chain_state.cuh"
 
 namespace sdv {
 
@@ -1647,6 +1649,84 @@ int sdv_bin_decode_verify(sdv_handle *h, int *redone)
     const int rc = decode_frames_impl(h, &c, h->lazy_luma, h->lazy_n, h->lazy_H, h->lazy_W, h->lazy_stride, h->lazy_recs, h->lazy_aux, h->lazy_stream);
     if(rc) return rc;
     if(redone) *redone = 1;
+    return SDV_OK;
+}
+
+// ---- the open file of the line decode as a blob (layout: CS_* in chain_state.cuh)
+static_assert(sizeof(sdv_bin_preset)==32, "blob layout of the fine settings");
+
+int sdv_bin_chain_state_bytes(void) { return CS_BYTES; }
+
+int sdv_bin_chain_state_save(sdv_handle *h, int pcm_type, void *state_dev, void *cuda_stream)
+{
+    if(!h) return SDV_ERR_ARG;
+    if(!state_dev||((uintptr_t)state_dev%4)) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_save: null or misaligned state buffer", cudaSuccess);
+    if(h->lazy_pending) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_save: the previous call was lazy (reserved[2] bit 1): call sdv_bin_decode_verify first", cudaSuccess);
+    int kind, H, W, mode, dup;
+    const void *ctx;
+    if((pcm_type==SDV_TYPE_STC007)||(pcm_type==SDV_TYPE_M2))
+    {
+        if(!h->chain_open||(((h->chain_mode>>9)&1)!=((pcm_type==SDV_TYPE_M2) ? 1 : 0)))
+            return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_save: no open file of this PCM type on the handle", cudaSuccess);
+        kind = CS_KIND_STC; ctx = h->ctx; H = h->chain_H; W = h->chain_W; mode = h->chain_mode&0xFF; dup = (h->chain_mode>>8)&1;
+    }
+    else if((pcm_type==SDV_TYPE_PCM1)||(pcm_type==SDV_TYPE_PCM16X0))
+    {
+        if(!h->pcm_open||(h->pcm_type!=pcm_type))
+            return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_save: no open file of this PCM type on the handle", cudaSuccess);
+        kind = (pcm_type==SDV_TYPE_PCM1) ? CS_KIND_P1 : CS_KIND_X0; ctx = (kind==CS_KIND_P1) ? (const void *)h->p1_ctx : (const void *)h->x0_ctx;
+        H = h->pcm_H; W = h->pcm_W; mode = h->pcm_mode&0xFF; dup = (h->pcm_mode>>8)&1;
+    }
+    else return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_save: pcm_type", cudaSuccess);
+    CK(cudaSetDevice(h->device));
+    ChainBlobHdr hdr; memset(&hdr, 0, sizeof(hdr));
+    u8 *b = (u8 *)hdr.w;
+    cs_put32(b, CSH_MAGIC, CS_MAGIC); cs_put16(b, CSH_VERSION, CS_VERSION); cs_put16(b, CSH_TYPE, (u32)pcm_type); cs_put32(b, CSH_SIZE, CS_BYTES);
+    cs_put16(b, CSH_H, (u32)H); cs_put16(b, CSH_W, (u32)W); b[CSH_MODE] = (u8)mode; b[CSH_DUP] = (u8)dup; b[CSH_M2] = (pcm_type==SDV_TYPE_M2) ? 1 : 0;
+    sdv_bin_preset fine; sdv_bin_get_fine_settings(h, &fine);
+    memcpy(b+CSH_FINE, &fine, sizeof(fine));
+    chain_state_pack_kernel<<<1, 128, 0, (cudaStream_t)cuda_stream>>>(hdr, kind, ctx, (u32 *)state_dev);
+    h->acc_launches += 1;
+    CK(cudaGetLastError());
+    return SDV_OK;
+}
+
+int sdv_bin_chain_state_load(sdv_handle *h, const void *state_dev, void *cuda_stream)
+{
+    if(!h) return SDV_ERR_ARG;
+    if(!state_dev||((uintptr_t)state_dev%4)) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_load: null or misaligned state buffer", cudaSuccess);
+    if(h->lazy_pending) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_load: the previous call was lazy (reserved[2] bit 1): call sdv_bin_decode_verify first", cudaSuccess);
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    std::vector<u8> blob(CS_BYTES);
+    CK(cudaMemcpyAsync(blob.data(), state_dev, CS_BYTES, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const u8 *b = blob.data();
+    const int kind = cs_blob_kind(b);
+    if(kind<0) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_load: not a line-decode chain state of this version", cudaSuccess);
+    {   // canonical: the state it holds packs to the same bytes (history entries past the counts and unused bytes zero)
+        std::vector<u8> again(blob.begin(), blob.begin()+CS_HDR);
+        again.resize(CS_BYTES, 0);
+        if(kind==CS_KIND_STC) { std::unique_ptr<ChainCtx> x(new ChainCtx()); cs_unpack_stc(b, x.get()); cs_pack_stc(x.get(), again.data()); }
+        else if(kind==CS_KIND_P1) { std::unique_ptr<P1ChainCtx> x(new P1ChainCtx()); cs_unpack_p1(b, x.get()); cs_pack_p1(x.get(), again.data()); }
+        else { std::unique_ptr<X0ChainCtx> x(new X0ChainCtx()); cs_unpack_x0(b, x.get()); cs_pack_x0(x.get(), again.data()); }
+        if(memcmp(again.data(), b, CS_BYTES)) return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_load: the blob is not in canonical form", cudaSuccess);
+    }
+    sdv_bin_preset fine; sdv_bin_get_fine_settings(h, &fine);
+    if(memcmp(b+CSH_FINE, &fine, sizeof(fine)))
+        return fail(h, SDV_ERR_ARG, "sdv_bin_chain_state_load: the handle's fine settings differ from the ones the state was saved with", cudaSuccess);
+    const int type = (int)cs_get16(b, CSH_TYPE), H = (int)cs_get16(b, CSH_H), W = (int)cs_get16(b, CSH_W);
+    const int key_mode = (int)b[CSH_MODE]|((int)b[CSH_DUP]<<8);
+    void *ctx = (kind==CS_KIND_STC) ? (void *)h->ctx : ((kind==CS_KIND_P1) ? (void *)h->p1_ctx : (void *)h->x0_ctx);
+    if(kind==CS_KIND_STC) h->chain_open = 0; else h->pcm_open = 0;
+    if(kind==CS_KIND_STC) chain_state_unpack_kernel<CS_KIND_STC><<<1, 128, 0, st>>>((const u32 *)state_dev, ctx);
+    else if(kind==CS_KIND_P1) chain_state_unpack_kernel<CS_KIND_P1><<<1, 128, 0, st>>>((const u32 *)state_dev, ctx);
+    else chain_state_unpack_kernel<CS_KIND_X0><<<1, 128, 0, st>>>((const u32 *)state_dev, ctx);
+    h->acc_launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    if(kind==CS_KIND_STC) { h->chain_open = 1; h->chain_H = H; h->chain_W = W; h->chain_mode = key_mode|((int)b[CSH_M2]<<9); }
+    else { h->pcm_open = 1; h->pcm_type = type; h->pcm_H = H; h->pcm_W = W; h->pcm_mode = key_mode; }
     return SDV_OK;
 }
 

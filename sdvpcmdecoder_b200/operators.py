@@ -121,6 +121,27 @@ class VideoToDigital:
         self.handle.check(rc)
         return (recs, aux) if want_aux else recs
 
+    def saveState(self, out: torch.Tensor | None = None, stream=None, pcm_type: int | None = None) -> torch.Tensor:
+        """The open file of the line decode (what doBinarize(continue_file=True) would continue) as a canonical uint8 CUDA tensor
+        of sdv_bin_chain_state_bytes() bytes (sdv_bin_chain_state_save): equal states give equal bytes.  pcm_type (default: this
+        operator's) selects the STC-007 / M2 file or the PCM-1 / PCM-16x0 one.  No synchronisation."""
+        n = int(capi.lib().sdv_bin_chain_state_bytes())
+        if out is None:
+            out = torch.empty(n, dtype=torch.uint8, device=torch.device("cuda", self.handle.device))
+        out = _dev_u8(out)
+        assert out.numel() == n
+        t = self.pcm_type if pcm_type is None else int(pcm_type)
+        self.handle.check(capi.lib().sdv_bin_chain_state_save(self.handle.ptr, t, C.c_void_p(out.data_ptr()), _stream_ptr(stream)))
+        return out
+
+    def loadState(self, state: torch.Tensor, stream=None):
+        """Make [state] (from saveState, on any handle or device) the open file of its kind on this handle: the next
+        doBinarize(continue_file=True) with the saved PCM type, geometry, mode and duplicate check continues it exactly
+        (sdv_bin_chain_state_load).  The handle's fine settings must be the ones the state was saved with."""
+        state = _dev_u8(state)
+        assert state.numel() == int(capi.lib().sdv_bin_chain_state_bytes())
+        self.handle.check(capi.lib().sdv_bin_chain_state_load(self.handle.ptr, C.c_void_p(state.data_ptr()), _stream_ptr(stream)))
+
     def stats(self) -> dict:
         return self.handle.last_stats()
 

@@ -1,7 +1,8 @@
 """Frame-range sharding of a tape over the ranks of one node (one process per GPU, torch.distributed).
 
-The decode path shards by contiguous frame ranges.  Line decode needs nothing from the neighbours (each shard starts
-its VideoToDigital chain empty, exactly like the reference at file start); the STC-007 deinterleaver reads 112 lines
+The decode path shards by contiguous frame ranges.  The plain sharded line decode needs nothing from the neighbours (each
+shard starts its VideoToDigital chain empty, exactly like the reference at file start); decode_shard instead hands the chain
+state from shard to shard, so that the shards equal one call over the whole tape.  The STC-007 deinterleaver reads 112 lines
 ahead (7 x 16 lines, stc007datablock.h:44-58), so shard g needs the first 112 line records of shard g+1: one small
 point-to-point message per boundary (NCCL send/recv over NVLink on GPUs, gloo in the CPU tests).  The one thing that
 flows the other way is the stitcher's broken-block countdown: a BROKEN block near the end of shard g masks the first blocks
@@ -307,27 +308,136 @@ def stitch_shard(stitcher, recs: torch.Tensor, n_frames: int, lines_per_frame: i
         out = stitcher.doFrameReassembleAuto(run_recs, run_recs.shape[0] // H, H, file_start=(rank == 0), file_end=last, **stitch_kw)
         return out, (None if last else stitcher.saveState())
     out, end = run()
-    rounds, redone = [], 0
     if world == 1:
-        return out, {"warmup_frames": 0, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone}
+        return out, {"warmup_frames": 0, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": [], "redone": 0}
     # (4) verify / redo (nobody compares with rank 0's start or the last rank's end: placeholders of the blob's shape)
     if rank == 0:
         start = end
     if last:
         end = start
+
+    def redo(state):
+        nonlocal out
+        stitcher.loadState(state)
+        out, end = run()
+        return state if last else end
+    rounds, redone = settle_states(transport, start, end, redo, "stitcher state")
+    return out, {"warmup_frames": k, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone}
+
+
+def settle_states(transport, start: torch.Tensor, end: torch.Tensor, redo, what: str = "state"):
+    """The verify / redo rounds of a shard hand-off.  [start]: the state this rank's run started from, [end]: the state it ended
+    with (canonical blobs: equality is byte equality; placeholders of the same shape where nobody compares them).  Every round
+    all-gathers the (start, end) pairs; every rank g > 0 whose start differs from rank g-1's end calls redo(that end) -> its new
+    end state.  Rank 0 is exact, so after round r the first r+1 shards are final: at most [world] rounds.
+    Returns (rounds: the ranks redone in each round, the same list on every rank; redone: the redo calls of this rank)."""
+    rank, world = transport.rank, transport.world
+    rounds, redone = [], 0
+    if world == 1:
+        return rounds, redone
     for _ in range(world + 1):
         both = transport.all_gather(torch.stack([start, end]))
         bad = [g for g in range(1, world) if not torch.equal(both[g, 0], both[g - 1, 1])]
         if not bad:
-            return out, {"warmup_frames": k, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone}
+            return rounds, redone
         rounds.append(bad)
         if rank in bad:
             start = both[rank - 1, 1].clone()
-            stitcher.loadState(start)
-            out, end = run()
-            end = start if last else end
+            end = redo(start)
             redone += 1
-    raise RuntimeError("stitcher state hand-off did not settle")
+    raise RuntimeError(f"{what} hand-off did not settle")
+
+
+# ---- line decode (VideoToDigital.doBinarize) over frame shards, exact
+#
+# The plain sharded decode starts every shard with an empty chain, as the reference does at a file start; on a damaged tape the
+# records at a shard's head can then differ from one call over the whole tape (Tier-B fields, the words of lines that fail their
+# CRC, with ignore_crc the samples).  decode_shard makes the shards exact with the protocol of stitch_shard: rank g decodes the
+# [warmup] frames in front of its first frame as a new file (records thrown away), continues over its own frames from the chain
+# state that leaves, and the (start, end) chain states (VideoToDigital.saveState, canonical) are verified by settle_states.
+#
+# The chain forgets: its presets follow the last good line, the damper the last 9 lines, the frame average the last 16 frames.
+# DECODE_WARMUP_FRAMES is that 16-frame reach plus a margin -- a guess until measured on damaged tapes.
+
+DECODE_WARMUP_FRAMES = 20
+
+
+def decode_shard(v2d, luma: torch.Tensor, transport, warmup: int = DECODE_WARMUP_FRAMES, edges=None, want_aux: bool = False):
+    """Line decode of this rank's frames [a, b) = frame_range(n_frames, rank, world) so that the shards' records (and aux)
+    concatenate to one doBinarize call over the whole tape, in every format.
+
+    v2d: a VideoToDigital on this rank's handle (PCM type, mode, duplicate check and fine settings as for the whole tape; one
+    chain segment); luma: CUDA uint8 [b-a, H, W], this rank's frames; transport: DistTransport or LocalTransport rank; edges:
+    world+1 frame indices [0, a_1, .., n_frames] for shards other than frame_range's (n_frames is then edges[-1]; without edges
+    it is the sum of the shards' frame counts, gathered).
+    Steps: (1) receive the luma of the [warmup] frames before a from rank-1 (passed along when shards are shorter); (2) decode
+    them as a new file, records discarded: the chain state this leaves is the guess at a (exact when the warm-up reaches frame
+    0); (3) continue over [a, b), save the end state; (4) settle_states: ranks whose start differs from their predecessor's end
+    load that end and decode again.  Rank 0 decodes from a file start.  warmup must be >= 1 on ranks > 0: a file start is no
+    state to continue (frame 0 carries the NEW_FILE line).
+    The STC-007 halo (the first 112 records of rank g+1) is final only when this returns: exchange it afterwards, not from
+    doBinarize's on_first_frame hook.
+    Returns (records, stats) or ((records, aux), stats); stats as stitch_shard's (warmup_frames, warmup_s, total_s, rounds,
+    redone) plus save_s and verify_s (time spent saving states and in the verify / redo rounds)."""
+    import time
+    rank, world = transport.rank, transport.world
+    n_own = luma.shape[0]
+    if edges is None:
+        counts = transport.all_gather(torch.tensor([n_own], dtype=torch.int64, device=luma.device)).view(-1).tolist()
+        edges = [0]
+        for c in counts:
+            edges.append(edges[-1] + int(c))
+    n_frames = edges[-1]
+    if len(edges) != world + 1 or edges[0] != 0 or any(edges[g + 1] <= edges[g] for g in range(world)):
+        raise ValueError("every shard needs at least one frame, and the shards must cover the tape")
+    a, b = edges[rank], edges[rank + 1]
+    if n_own != b - a:
+        raise ValueError("luma must hold this rank's frames")
+    if rank > 0 and warmup < 1:
+        raise ValueError("decode_shard needs warmup >= 1 on ranks > 0: a file start is no chain state to continue")
+    if getattr(v2d, "chain_segments", 1) > 1:
+        raise ValueError("decode_shard decodes one file: chain_segments must be 1")
+    t0 = time.perf_counter()
+    # (1) luma of the frames in front
+    k = min(warmup, a)
+    head = luma.new_empty((k,) + tuple(luma.shape[1:]))
+    if rank > 0:
+        transport.recv(head, rank - 1)
+    if rank < world - 1:
+        k_next = min(warmup, b)
+        transport.send(torch.cat([head, luma])[k + (b - a) - k_next:], rank + 1)
+    # (2) warm-up
+    t_save = 0.0
+    if rank > 0:
+        v2d.doBinarize(head)
+        ts = time.perf_counter()
+        start = v2d.saveState()
+        t_save += time.perf_counter() - ts
+    t_warm = time.perf_counter() - t0
+
+    # (3) the shard
+    def run():
+        nonlocal t_save
+        out = v2d.doBinarize(luma, want_aux=want_aux, continue_file=(rank > 0))
+        ts = time.perf_counter()
+        end = v2d.saveState()
+        t_save += time.perf_counter() - ts
+        return out, end
+    out, end = run()
+    if rank == 0:
+        start = end
+
+    # (4) verify / redo
+    def redo(state):
+        nonlocal out
+        v2d.loadState(state)
+        out, e = run()
+        return e
+    tv = time.perf_counter()
+    rounds, redone = settle_states(transport, start, end, redo, "line-decode chain state")
+    t_verify = time.perf_counter() - tv
+    return out, {"warmup_frames": k, "warmup_s": t_warm, "total_s": time.perf_counter() - t0, "rounds": rounds, "redone": redone,
+                 "save_s": t_save, "verify_s": t_verify}
 
 
 def bind_to_gpu_numa_node(device_index: int):
