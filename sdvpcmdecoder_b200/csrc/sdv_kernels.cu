@@ -10,7 +10,8 @@
 //                          pass cannot take: the first frame and every frame with a line that fails the preset decode.
 //                          One block (or one block per segment); warps look ahead with the preset decode, the whole block
 //                          runs the full Binarizer on a failing line, thread 0 advances the chain.
-//   stc007_deint_kernel  (here; stc007_deint.cuh) : one thread per data block, per-warp tiles staged through shared
+//   stc007_deint_kernel  (here; stc007_deint.cuh) : one thread per data block (two adjacent blocks per lane, packed in
+//                          16-bit halves, in the standard setting), per-warp tiles staged through shared
 //                          memory, P/Q correction in registers, samples + flags out; broken_window_kernel for the
 //                          128-block unsafe windows; stc007_seam_kernel for the field-seam padding sweep.
 //   pcm1_* / pcm16x0_*   (pcm1_kernels.cuh, pcm16x0_kernels.cuh, pcm1_stitch.cuh, pcm16x0_stitch.cuh, *_deint.cuh) :
@@ -419,7 +420,9 @@ __device__ __forceinline__ void block_store(const Block &blk, bool unsafe, long 
 // with itself, and each lane then finishes 4 blocks.  No block-wide barrier: warps overlap each other's load latency.
 enum { DEINT_WARPS = 8, DEINT_TILE = 128, DEINT_TLINES = DEINT_TILE+112, DEINT_THREADS = DEINT_WARPS*32, DEINT_CTA_BLOCKS = DEINT_WARPS*DEINT_TILE };
 
-__global__ void __launch_bounds__(DEINT_THREADS) stc007_deint_kernel(DeintParams p)
+// PAIR: the standard setting with samples and flags only, an even first block and 8- / 4-byte aligned sample / flag buffers
+// (deint_pair_applies): each lane finishes two adjacent blocks at once.
+template<bool PAIR> __global__ void __launch_bounds__(DEINT_THREADS) stc007_deint_kernel(DeintParams p)
 {
     __shared__ u16 s_wall[DEINT_WARPS][8][DEINT_TLINES];    // word-major: lane t reads s_w[k][t+16k], consecutive lanes consecutive addresses
     const int warp = threadIdx.x>>5, lane = threadIdx.x&31;
@@ -508,6 +511,89 @@ __global__ void __launch_bounds__(DEINT_THREADS) stc007_deint_kernel(DeintParams
         }
     }
     __syncwarp();
+    // The standard setting with samples and flags only: each lane takes blocks s and s+1 (s even) at once, as packed word pairs
+    // (stc007_deint.cuh, deint_pair_std14) -- word k of lines s+16k and s+1+16k is one 32-bit shared load, their trusted bits
+    // one 2-bit field of the ballot windows -- and stores 24 bytes of samples and 12 of flags.  Pairs it does not cover, and a
+    // block whose partner lies past the tile or the stream, go through deint_block_std14() one by one.
+    if constexpr(PAIR)
+    {
+        const int n_here = (int)(((long long)p.tile_len<p.n_blocks-b0) ? (long long)p.tile_len : (p.n_blocks-b0));
+        u32 lw[(DEINT_TLINES+31)/32-1];     // the window words from this half-warp's first line on: lanes 16..31 start 32 lines later
+#pragma unroll
+        for(int i=0;i<(DEINT_TLINES+31)/32-1;i++) lw[i] = (lane<16) ? okw[i] : okw[i+1];
+        // Both pairs of the lane first, as two independent branch-free chains; then their stores, or the one-block path
+        u32 d[DEINT_TILE/64][6], f[DEINT_TILE/64][3], bnp[DEINT_TILE/64], okf[DEINT_TILE/64][4];
+        bool cov[DEINT_TILE/64];
+#pragma unroll
+        for(int jt=0;jt<DEINT_TILE/64;jt++)
+        {
+            const int s = 2*lane+64*jt;
+            u32 w[8];       // (lines s+16k, s+1+16k < DEINT_TLINES: always inside the staged tile)
+#pragma unroll
+            for(int k=0;k<8;k++) w[k] = *(const u32 *)&s_w[k][s+16*k];
+            // bits 0 / 1: line s+32m / s+1+32m (word 2m of blocks s / s+1); bits 16 / 17: 16 lines on (word 2m+1)
+#pragma unroll
+            for(int m=0;m<4;m++) okf[jt][m] = __funnelshift_r(lw[2*jt+m], lw[2*jt+m+1], 2*lane);
+            BlockPair bp;
+            cov[jt] = deint_pair_std14(w, okf[jt], &bp);
+            pair_samples(&bp, d[jt]);
+            pair_flags(&bp, f[jt]);
+            bnp[jt] = pair_broken_ns(&bp);
+        }
+#pragma unroll
+        for(int jt=0;jt<DEINT_TILE/64;jt++)
+        {
+            const int s = 2*lane+64*jt;
+            const long long b = b0+s;
+            u32 bns = 0;    // bit h: block s+h is BROKEN and not silent
+            if(cov[jt]&&(s+1<n_here))
+            {
+                uint2 *sd = (uint2 *)(p.samples+b*6);
+                sd[0] = make_uint2(d[jt][0], d[jt][1]); sd[1] = make_uint2(d[jt][2], d[jt][3]); sd[2] = make_uint2(d[jt][4], d[jt][5]);
+                u32 *fd = (u32 *)(p.sflags+b*6);
+                fd[0] = f[jt][0]; fd[1] = f[jt][1]; fd[2] = f[jt][2];
+                bns = bnp[jt];
+            }
+            else
+            {
+                for(int h=0;h<2;h++)
+                {
+                    if(s+h>=n_here) break;
+                    BlockIn in; in.ok = 0;
+#pragma unroll
+                    for(int k=0;k<8;k++)
+                    {
+                        const int ln = s+h+16*k;
+                        in.w[k] = s_w[k][ln]; in.sw[k] = s_w[7][ln];
+                        in.ok |= (u8)(((okf[jt][k>>1]>>(16*(k&1)+h))&1u)<<k);
+                    }
+                    Block blk;
+                    deint_block_std14(&blk, &in);
+                    blk.m2 = 0;
+                    if((blk.audio_state==SDV_AUD_BROKEN)&&!blk_silent(&blk)) bns |= 1u<<h;
+                    block_store(blk, false, b+h, p.blocks, p.samples, p.sflags);
+                }
+            }
+            if(p.atomic_bits)
+            {
+                if(p.broken_bits)
+                    for(int h=0;h<2;h++)
+                        if((bns>>h)&1u) { atomicOr(&p.broken_bits[(b+h)>>5], 1u<<(u32)((b+h)&31)); p.broken_sum[(b+h)>>10] = 1; }
+            }
+            else
+            {   // blocks 64jt..+31 are lanes 0..15, the next 32 lanes 16..31: lanes 0 and 16 write the two words
+                const u32 v = bns<<((2*lane)&31);
+                const u32 bal0 = __reduce_or_sync(0xFFFFFFFFu, (lane<16) ? v : 0u), bal1 = __reduce_or_sync(0xFFFFFFFFu, (lane<16) ? 0u : v);
+                const u32 bal = (lane<16) ? bal0 : bal1;
+                if(((lane&15)==0)&&(b<p.n_blocks))
+                {
+                    if(p.broken_bits) p.broken_bits[b>>5] = bal;
+                    if(bal&&p.broken_sum) p.broken_sum[b>>10] = 1;
+                }
+            }
+        }
+        return;
+    }
     for(int jt=0;jt<DEINT_TILE/32;jt++)
     {
         const int s = lane+32*jt;
@@ -1772,6 +1858,19 @@ static int run_windows(sdv_handle *h, const DeintScratch &sc, WindowParams &wp, 
     return SDV_OK;
 }
 
+// stc007_deint_kernel<true> wherever it applies: the standard setting without the M2 expansion, no block records, both output
+// buffers aligned for the 8-byte sample / 4-byte flag stores of a pair, and every tile starting on an even block.
+static bool deint_pair_applies(const DeintParams &p)
+{
+    return deint_cfg_is_std14(p.cfg)&&(!p.cfg.m2)&&(!p.blocks)&&p.samples&&p.sflags&&((((uintptr_t)p.samples)&7u)==0)
+           &&((((uintptr_t)p.sflags)&3u)==0)&&((p.tile_base&1)==0)&&((p.tile_stride&1)==0);
+}
+static void launch_deint(const DeintParams &p, unsigned grid, cudaStream_t st)
+{
+    if(deint_pair_applies(p)) stc007_deint_kernel<true><<<grid, DEINT_THREADS, 0, st>>>(p);
+    else stc007_deint_kernel<false><<<grid, DEINT_THREADS, 0, st>>>(p);
+}
+
 static int run_deint(sdv_handle *h, const sdv_deint_config *cfg, const AsmMap &map, long long n_blocks,
                      sdv_block_rec *blocks_dev, int16_t *samples_dev, uint8_t *sample_flags_dev, cudaStream_t st)
 {
@@ -1805,7 +1904,7 @@ static int run_deint(sdv_handle *h, const sdv_deint_config *cfg, const AsmMap &m
             DeintParams q = p;
             q.n_blocks = (head<n_blocks) ? head : n_blocks;
             q.n_tiles = (int)((q.n_blocks+DEINT_TILE-1)/DEINT_TILE);
-            stc007_deint_kernel<<<(unsigned)((q.n_tiles+DEINT_WARPS-1)/DEINT_WARPS), DEINT_THREADS, 0, st>>>(q);
+            launch_deint(q, (unsigned)((q.n_tiles+DEINT_WARPS-1)/DEINT_WARPS), st);
             h->acc_launches += 1;
         }
         const int n_rest = fd.n_frames-fd.f_from;
@@ -1813,7 +1912,7 @@ static int run_deint(sdv_handle *h, const sdv_deint_config *cfg, const AsmMap &m
         {
             DeintParams q = p;
             q.tile_base = head+(2*fd.lpf-112); q.tile_stride = 2*fd.lpf; q.tile_len = 112; q.n_tiles = n_rest;
-            stc007_deint_kernel<<<(unsigned)((q.n_tiles+DEINT_WARPS-1)/DEINT_WARPS), DEINT_THREADS, 0, st>>>(q);
+            launch_deint(q, (unsigned)((q.n_tiles+DEINT_WARPS-1)/DEINT_WARPS), st);
             h->acc_launches += 1;
         }
     }
@@ -1821,7 +1920,7 @@ static int run_deint(sdv_handle *h, const sdv_deint_config *cfg, const AsmMap &m
     {
         if(windows) CK(cudaMemsetAsync(sc.sum, 0, (size_t)((n_blocks+1023)>>10), st));
         const unsigned grid = (unsigned)((n_blocks+DEINT_CTA_BLOCKS-1)/DEINT_CTA_BLOCKS);
-        stc007_deint_kernel<<<grid, DEINT_THREADS, 0, st>>>(p);
+        launch_deint(p, grid, st);
         h->acc_launches += 1;
     }
     cudaEventRecord(h->ev[3], st);

@@ -439,6 +439,175 @@ SDV_HD void deint_block_std14(Block *blk, const BlockIn *in)
     blk->line_crc = (u8)crc; blk->word_valid = (u8)valid; blk->resolution = RES_14BIT; blk->audio_state = (u8)state;
 }
 
+// ---- Two adjacent blocks of the standard setting in one instruction stream.  Block s sits in the low 16-bit half of every
+// word, block s+1 in the high half ("packed").  A pair in which each block has at most one untrusted line -- the clean tape:
+// the uncaptured lines of a field are 16 lines apart from nothing else in a block -- is finished here with masks, without a
+// branch; any other pair goes to deint_block_std14() block by block (deint_pair_std14() returns false).
+
+// __byte_perm(x, y, s) without the sign modes: byte i of the result = byte (s>>4i)&7 of the 8-byte value y:x.
+SDV_HD u32 prmt(u32 x, u32 y, u32 s)
+{
+#if defined(__CUDA_ARCH__)
+    return __byte_perm(x, y, s);
+#else
+    const u64 v = ((u64)y<<32)|x;
+    u32 r = 0;
+    for(int i=0;i<4;i++) r |= (u32)((v>>(8*((s>>(4*i))&7u)))&0xFFu)<<(8*i);
+    return r;
+#endif
+}
+#if defined(__CUDA_ARCH__)
+// PTX prmt in its default mode: a selector nibble with bit 3 set replicates the sign of the selected byte over the result byte
+// (__byte_perm() drops that bit).
+__device__ __forceinline__ u32 prmt_sign(u32 x, u32 s)
+{
+    u32 r;
+    asm("prmt.b32 %0, %1, 0, %2;" : "=r"(r) : "r"(x), "r"(s));
+    return r;
+}
+#endif
+// Bit 15 / bit 31 -> 0xFFFF in the low / high half.
+SDV_HD u32 msb_to_halves(u32 h)
+{
+#if defined(__CUDA_ARCH__)
+    return prmt_sign(h, 0xBB99);                // every byte the sign of byte 1 / byte 3
+#else
+    return ((h>>15)&0x10001u)*0xFFFFu;
+#endif
+}
+// 0xFFFF in each half that is not zero.
+SDV_HD u32 nz_halves(u32 v) { return msb_to_halves((((v&0x7FFF7FFFu)+0x7FFF7FFFu)|v)&0x80008000u); }
+// The line-trusted masks of words 2m (hi = 0) and 2m+1 (hi = 1) from the 2-bit fields of okf: bits 0 / 1 = word 2m of block
+// s / s+1, bits 16 / 17 = word 2m+1.  One multiplication puts the four bits on the sign bits of the four bytes.
+SDV_HD u32 pair_okmask(u32 okf, int hi)
+{
+    const u32 y = (okf&0x00030003u)*0x4080u;
+#if defined(__CUDA_ARCH__)
+    return prmt_sign(y, hi ? 0xBBAA : 0x9988);
+#else
+    const u32 a = (y>>(7+16*hi))&1u, b = (y>>(15+16*hi))&1u;
+    return (a ? 0x0000FFFFu : 0u)|(b ? 0xFFFF0000u : 0u);
+#endif
+}
+// q_of_words() on both halves.  The low 14 bits of every shifted word stay in their half once the bits pushed past bit 13
+// (and, in the high half, the low half's carried-over bits) are masked off; those top bits -- six at most -- are gathered
+// shifted down by 14, and the sum is folded once as in q_of_words().
+SDV_HD u32 q_of_word_pairs(const u32 *w)
+{
+    u32 lo = 0, top = 0;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<6;k++)
+    {
+        const int s = 6-k;
+        const u32 low_s = (1u<<s)-1u;
+        lo ^= (w[k]<<s)&(0x3FFF3FFFu&~(low_s<<16));
+        top ^= (w[k]>>(14-s))&(low_s*0x10001u);
+    }
+    return lo^top^(top<<8);
+}
+
+struct BlockPair
+{
+    u32 words[8];       // packed block words after correction / regeneration
+    u32 okm[8];         // 0xFFFF per half: the line of word k is trusted (line_crc of a block that is not BROKEN)
+    u32 broken;         // 0xFFFF per half: BROKEN
+    u32 fixed;          // 0xFFFF per half: an audio word was put right by P (SDV_AUD_FIX_P)
+};
+
+// deint_block_std14() for blocks s and s+1: w = packed words 0..7, okf[m] = the 2-bit fields of words 2m and 2m+1 (see
+// pair_okmask; other bits are ignored).  With at most one untrusted word per block the cases of deint_block_std14() are
+//   audio word i untrusted: w_i ^= Sp, then the Q check on the corrected words;
+//   P untrusted: the Q check, P regenerated;  Q untrusted: the P check, Q regenerated;  none: the P and Q checks,
+// which is: correct by Sp wherever an audio word is untrusted, then BROKEN = (Q trusted and Sq of the corrected words != 0)
+// or (P and all audio words trusted and Sp != 0).  Returns false when a block has two or more untrusted words.
+SDV_HD bool deint_pair_std14(const u32 *w, const u32 *okf, BlockPair *r)
+{
+    u32 o[8];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int m=0;m<4;m++) { o[2*m] = pair_okmask(okf[m], 0); o[2*m+1] = pair_okmask(okf[m], 1); }
+    u32 any = 0, two = 0;           // per half: some / a second untrusted word
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<8;k++) { two |= any&~o[k]; any |= ~o[k]; }
+    const u32 sp = w[0]^w[1]^w[2]^w[3]^w[4]^w[5]^w[W_P0];
+    u32 c[6];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<6;k++) c[k] = w[k]^(sp&~o[k]);
+    const u32 cq = q_of_word_pairs(c);
+    const u32 sq = cq^w[W_Q0];
+    const u32 aud_ok = o[0]&o[1]&o[2]&o[3]&o[4]&o[5];
+    const u32 broken = nz_halves((sq&o[W_Q0])|(sp&aud_ok&o[W_P0]));
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<6;k++) r->words[k] = c[k];
+    // a regenerated word only where the block is not BROKEN; an untrusted P means no audio word was corrected
+    const u32 reg_p = ~o[W_P0]&~broken, reg_q = ~o[W_Q0]&~broken;
+    r->words[W_P0] = (w[W_P0]&~reg_p)|((sp^w[W_P0])&reg_p);
+    r->words[W_Q0] = (w[W_Q0]&~reg_q)|(cq&reg_q);
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<8;k++) r->okm[k] = o[k];
+    r->broken = broken;
+    r->fixed = ~aud_ok;
+    return two==0;          // (decided last: nothing above waits for it)
+}
+
+// The six samples of each block (words << 2 in 14-bit mode), as the 24 bytes they take in the sample stream.
+SDV_HD void pair_samples(const BlockPair *r, u32 *d /*[6]*/)
+{
+    u32 s[6];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<6;k++) s[k] = (r->words[k]<<2)&0xFFFCFFFCu;
+    d[0] = prmt(s[0], s[1], 0x5410); d[1] = prmt(s[2], s[3], 0x5410); d[2] = prmt(s[4], s[5], 0x5410);
+    d[3] = prmt(s[0], s[1], 0x7632); d[4] = prmt(s[2], s[3], 0x7632); d[5] = prmt(s[4], s[5], 0x7632);
+}
+// blk_output_flags() of both blocks as the 12 flag bytes: a block that is not BROKEN has all words valid here, so a sample's
+// flags are BLOCK_OK | WORD_VALID, and WORD_FIXED where its line was trusted; a BROKEN block's are 0.
+SDV_HD void pair_flags(const BlockPair *r, u32 *f /*[3]*/)
+{
+    u32 g[6];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for(int k=0;k<6;k++) g[k] = ~r->broken&((r->okm[k]&(SDV_SF_WORD_FIXED*0x10001u))|((SDV_SF_BLOCK_OK|SDV_SF_WORD_VALID)*0x10001u));
+    const u32 g01 = prmt(g[0], g[1], 0x6240), g23 = prmt(g[2], g[3], 0x6240), g45 = prmt(g[4], g[5], 0x6240);     // [A_k A_k+1 B_k B_k+1]
+    f[0] = prmt(g01, g23, 0x5410); f[1] = prmt(g45, g01, 0x7610); f[2] = prmt(g23, g45, 0x7632);
+}
+// Bit 0 / 1: block s / s+1 is BROKEN and not silent (may open a countdown window).
+SDV_HD u32 pair_broken_ns(const BlockPair *r)
+{
+    const u32 loud = nz_halves((r->words[0]|r->words[1]|r->words[2]|r->words[3]|r->words[4]|r->words[5])&0x3FFF3FFFu);
+    const u32 b = r->broken&loud;
+    return (b&1u)|((b>>15)&2u);
+}
+// The two Blocks deint_block_std14() would give (what the pair carries in packed form).
+SDV_HD void pair_unpack(const BlockPair *r, Block *a, Block *b)
+{
+    Block *blk[2] = { a, b };
+    for(int h=0;h<2;h++)
+    {
+        const int sh = 16*h;
+        u32 ok = 0;
+        for(int k=0;k<8;k++) { blk[h]->words[k] = (u16)(r->words[k]>>sh); ok |= ((r->okm[k]>>sh)&1u)<<k; }
+        const bool broken = (r->broken>>sh)&1u;
+        blk[h]->line_crc = broken ? 0 : (u8)ok;
+        blk[h]->word_valid = broken ? 0 : 0xFF;
+        blk[h]->resolution = RES_14BIT;
+        blk[h]->audio_state = broken ? SDV_AUD_BROKEN : (((r->fixed>>sh)&1u) ? SDV_AUD_FIX_P : SDV_AUD_ORIG);
+    }
+}
+
 SDV_HD bool deint_cfg_is_std14(DeintCfg cfg) { return (cfg.res_mode==SDV_RES_MODE_14BIT)&&cfg.force_check&&cfg.p_corr&&cfg.q_corr; }
 SDV_HD void deint_dispatch(Block *blk, const BlockIn *in, DeintCfg cfg)
 {
